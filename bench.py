@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path on the BASELINE.json workload, one JSON line on stdout (rank 0).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one full log-likelihood evaluation of the workload (K1 P(t) tables for every branch x class,
@@ -10,6 +10,8 @@ per-shard scalars).  ``value`` = CLV updates per second (one update = one (node,
 an internal node's conditional likelihood vector, SURVEY.md 8d), whole job, inputs resident in HBM.
 ``e2e`` = the same through the C-ABI call sequence of one optimiser step with HOST buffers: branch lengths and the
 model eigensystem go host->device, log L (and derivatives) come back device->host, inside the timed region.
+``--dump-outputs DIR`` writes what the last timed step returned (lnl, and d1 / d2 where the workload asks for them) as
+DIR/<name>.npy in float64; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -25,6 +27,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it
 # stdout carries exactly one JSON line: keep NCCL's banner ("NCCL version ...") and any debug output on stderr
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
 
@@ -68,6 +71,22 @@ def emit(line):
     _claim_stdout()
     _JSON_OUT.write(json.dumps(line) + "\n")
     _JSON_OUT.flush()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """d/<name>.npy (float64) for every array, DUMP_BYTES in all: an array over its share is replaced by the same seeded sample
+    of its flattened entries on every run."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // 8 // len(arrays)
+    for name, x in arrays.items():
+        x = np.asarray(x, np.float64)
+        if x.size > share:
+            x = x.ravel()[np.sort(np.random.default_rng(0).choice(x.size, share, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), x)
+    log("outputs of the last timed step written to %s: %s" % (d, ", ".join(sorted(arrays))))
 
 
 class ClockSampler:
@@ -371,6 +390,14 @@ def run_points(a, w, rank, world, local, K, W, metric, config):
         e.eval_device(1, out.data_ptr(), stream.cuda_stream)
     ev1.record(stream)
     barrier()
+    if a.dump_outputs:
+        lnl_pts = out.view(npts, 1 + 2 * nn)[:, 0].cpu().numpy()
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, lnl_pts)
+            lnl_pts = np.concatenate(parts)
+        if rank == 0:
+            dump_outputs(a.dump_outputs, {"lnl": lnl_pts})
     ms = ev0.elapsed_time(ev1)
     st = e.stats()
     log("[rank %d] timed region done: %.3f ms/step, P(t) %.3f ms, pruning %.3f ms" % (rank, ms / K, st["pt_ms_sum"] / K, st["prune_ms_sum"] / max(1, st["prune_count"])))
@@ -517,7 +544,11 @@ def main():
                     help="chromosome workload: redraw parameter points whose eigen form misses the generator (the round-1 sample)")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling job timed after the strong one")
     ap.add_argument("--profile", action="store_true", help="1 warm-up + 1 timed step, no e2e / CPU legs (for ncu only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float64, at most 64 MB in all)")
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     w = dict(WORKLOADS[a.workload])
     if a.patterns:
@@ -566,6 +597,8 @@ def main():
         if a.warmup:
             ref_cpu.eval_raw(reps=max(1, a.warmup), **args)
         r = ref_cpu.eval_raw(reps=K, **args)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {"lnl": [r["lnl"]], "d1": r["d1"], "d2": r["d2"]} if w["derivs"] else {"lnl": [r["lnl"]]})
         dt = r["total_seconds"]
         upd = tree.n_internal * n * w["C"] * w["S"]
         val = upd * K / dt
@@ -631,6 +664,9 @@ def main():
         step_device()
     ev1.record(stream)
     barrier()
+    if a.dump_outputs and rank == 0:
+        res = out.cpu().numpy()          # every rank holds the whole alignment's result row
+        dump_outputs(a.dump_outputs, {"lnl": res[:1], "d1": res[1:1 + nn], "d2": res[1 + nn:]} if w["derivs"] else {"lnl": res[:1]})
     ms = ev0.elapsed_time(ev1)
     log("[rank %d] timed region done: %.3f ms/step" % (rank, ms / K))
     st = e.stats()

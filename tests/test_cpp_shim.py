@@ -5,6 +5,7 @@ flattening, site patterns) agree with the oracle.  GPU part: tests/cpp/test_like
 test_likelihood.cpp / test_likelihood_clock.cpp rewritten against the shim -- exits 0, and the values it prints for
 the other state spaces match the oracle."""
 import json
+import os
 import pathlib
 import subprocess
 
@@ -33,9 +34,11 @@ def compile_cpp(name, built_lib):
 
 
 @pytest.fixture(scope="module")
-def host_doc(built_lib):
+def host_doc(built_lib, tmp_path_factory):
     exe = compile_cpp("shim_host", built_lib)
-    return json.loads(subprocess.check_output([str(exe)]))
+    # the file readers' inputs go to a directory of this run, not to a /tmp shared with other users
+    env = dict(os.environ, BPPGPU_TEST_TMP=str(tmp_path_factory.mktemp("shim_io")))
+    return json.loads(subprocess.check_output([str(exe)], env=env))
 
 
 def test_shim_and_reference_style_test_compile(built_lib):

@@ -466,4 +466,8 @@ class Engine:
     def stats(self):
         s = Stats()
         _check(lib().bppgpu_get_stats(self._h, C.byref(s)))
-        return {k: getattr(s, k) for k, _ in Stats._fields_}
+        out = {k: getattr(s, k) for k, _ in Stats._fields_}
+        nf = C.c_int32(0)
+        _check(lib().bppgpu_get_frontier_nodes(self._h, C.byref(nf)))
+        out["w4c_frontier_nodes"] = nf.value
+        return out

@@ -88,8 +88,11 @@ static int ilog2(int v) {
 // op stays the reference's son order (RHomogeneousTreeLikelihood.cpp:827-861).
 // reg_slot (walk4c): a push whose lifetime contains no other push -- the sibling evaluated next has label 1, i.e. is a
 // caterpillar -- goes to the kernel's register slot (dst_slot = -2, child kind CHILD_RSLOT) instead of a shared-memory slot.
-static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg_slot = false) {
+// folded (walk4c): nodes the program treats as tips (CHILD_TIP, idx -1): cherries whose rows the table pass computes.
+static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg_slot = false,
+                          const std::vector<char>* folded = nullptr) {
   const int nn = e->nn;
+  auto is_leaf = [&](int n) { return e->leaf_slot[n] >= 0 || (folded && (*folded)[n]); };
   std::vector<int> label(nn, 0);
   // node ids are arbitrary: compute labels by an explicit post-order
   std::vector<int> order;
@@ -117,7 +120,7 @@ static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg
     std::vector<int> ls;
     for (int j = 0; j < nc; ++j) {
       int ch = e->children[e->child_off[n] + j];
-      if (e->leaf_slot[ch] < 0) ls.push_back(label[ch]);
+      if (!is_leaf(ch)) ls.push_back(label[ch]);
     }
     std::sort(ls.begin(), ls.end(), std::greater<int>());
     int lab = 1;
@@ -137,7 +140,7 @@ static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg
     std::vector<int> internal;
     for (int j = 0; j < nc; ++j) {
       int ch = e->children[e->child_off[n] + j];
-      if (e->leaf_slot[ch] < 0) internal.push_back(ch);
+      if (!is_leaf(ch)) internal.push_back(ch);
     }
     std::stable_sort(internal.begin(), internal.end(), [&](int a, int b) { return label[a] > label[b]; });
     for (size_t i = 0; i < internal.size(); ++i) {
@@ -168,7 +171,7 @@ static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg
       int ch = e->children[e->child_off[n] + j];
       Child c{};
       c.pnode = ch;
-      if (e->leaf_slot[ch] >= 0) {
+      if (is_leaf(ch)) {
         c.kind = CHILD_TIP;
         c.idx = e->leaf_slot[ch];
       } else if (all_keep) {
@@ -786,23 +789,47 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
   if (e->path == PATH_WALK4 && !e->keep && !(getenv("BPPGPU_WALK4C") && atoi(getenv("BPPGPU_WALK4C")) == 0)) {
     // walk4c: the same walk with leaf pushes in the register slot, tables cut into fixed-size chunks in walk order, the
     // program (descriptor words + chunk records) in the kernel-parameter block
-    build_program(e, e->prog4c, false, true);
-    const int blk_int = C * 128, blk_tip = C * e->ncodes * 32;
+    const int W = e->ncodes * e->ncodes;
+    const int blk_int = C * 128, blk_tip = C * e->ncodes * 32, blk_wide = w4c_wide_block_bytes(C, W);
+    // chunk geometry: bytes of tables and tip-code rows per ring stage (tuning knobs; a stage must hold the largest op)
+    int CH = getenv("BPPGPU_WALK4_CH") ? std::max(1024, atoi(getenv("BPPGPU_WALK4_CH")) & ~127) : 8192;
+    // Folded cherries: a cherry whose father is binary becomes a wide tip of the father (walk4c_kernels.cuh), its op leaves
+    // the walk.  W <= 64 code pairs keep a row code in one byte and a wide block (C W 36 bytes) small next to the chunk; a
+    // father whose op would outgrow the chunk keeps its second cherry as it is.  The fathers stay binary, so every op with a
+    // wide tip is one of the binary shapes.  BPPGPU_W4C_FRONTIER=0 folds none (the program of the unfolded walk).
+    e->w4c_cherry.assign(nn, 0);
+    if (W <= kW4cMaxWideCodes && !(getenv("BPPGPU_W4C_FRONTIER") && atoi(getenv("BPPGPU_W4C_FRONTIER")) == 0)) {
+      auto sons = [&](int n) { return e->child_off[n + 1] - e->child_off[n]; };
+      auto son = [&](int n, int j) { return e->children[e->child_off[n] + j]; };
+      auto cherry = [&](int n) { return sons(n) == 2 && e->leaf_slot[son(n, 0)] >= 0 && e->leaf_slot[son(n, 1)] >= 0; };
+      for (int f = 0; f < nn; ++f) {
+        if (sons(f) != 2) continue;
+        for (int j = 0; j < 2; ++j) e->w4c_cherry[son(f, j)] = cherry(son(f, j));
+        for (int j = 1; j >= 0; --j) {
+          int b = 0;
+          for (int k = 0; k < 2; ++k) {
+            const int ch = son(f, k);
+            b += e->w4c_cherry[ch] ? blk_wide : e->leaf_slot[ch] >= 0 ? blk_tip : blk_int;
+          }
+          if (b > CH) e->w4c_cherry[son(f, j)] = 0;
+        }
+      }
+    }
+    build_program(e, e->prog4c, false, true, &e->w4c_cherry);
+    auto child_bytes = [&](const Child& ch) { return ch.kind != CHILD_TIP ? blk_int : ch.idx >= 0 ? blk_tip : blk_wide; };
     int max_op = 0, max_tips_op = 0;
     bool ok = e->prog4c.nslots <= 63;
     for (const Op& op : e->prog4c.ops) {
       int b = 0, nt = 0;
       for (int j = 0; j < op.nchild; ++j) {
-        const bool tip = e->prog4c.childs[op.child_begin + j].kind == CHILD_TIP;
-        b += tip ? blk_tip : blk_int;
-        nt += tip;
+        const Child& ch = e->prog4c.childs[op.child_begin + j];
+        b += child_bytes(ch);
+        nt += ch.kind == CHILD_TIP;
       }
       max_op = std::max(max_op, b);
       max_tips_op = std::max(max_tips_op, nt);
       if (op.nchild > 6) ok = false;
     }
-    // chunk geometry: bytes of tables and tip-code rows per ring stage (tuning knobs; a stage must hold the largest op)
-    int CH = getenv("BPPGPU_WALK4_CH") ? std::max(1024, atoi(getenv("BPPGPU_WALK4_CH")) & ~127) : 8192;
     while (CH < max_op) CH *= 2;
     e->w4c_max_tips = getenv("BPPGPU_WALK4_MAXTIPS") ? std::max(1, std::min(31, atoi(getenv("BPPGPU_WALK4_MAXTIPS")))) : kW4cMaxTipsPerChunk;
     e->w4c_max_tips = std::max(e->w4c_max_tips, max_tips_op);
@@ -892,28 +919,34 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
       for (const Op& op : e->prog4c.ops) {
         int b = 0, nt = 0;
         for (int j = 0; j < op.nchild; ++j) {
-          const bool tip = e->prog4c.childs[op.child_begin + j].kind == CHILD_TIP;
-          b += tip ? blk_tip : blk_int;
-          nt += tip;
+          const Child& ch = e->prog4c.childs[op.child_begin + j];
+          b += child_bytes(ch);
+          nt += ch.kind == CHILD_TIP;
         }
         if (nops_in == 31 || used + (size_t)b > (size_t)CH || ntips_in + nt > e->w4c_max_tips) close_chunk();
         auto kind4c = [](int k) { return k == CHILD_TIP ? W4C_TIP : k == CHILD_SLOT ? W4C_SLOT : k == CHILD_RSLOT ? W4C_RSL : W4C_REG; };
         int shape = W4C_GENERIC;
         int order[8] = {0, 1, 2, 3, 4, 5, 6, 7};   // order in which the handler consumes the children's table blocks
-        unsigned jslot = 0;
+        unsigned jslot = 0, wide = 0;
         if (op.nchild == 2) {
           const Child& ca = e->prog4c.childs[op.child_begin];
           const Child& cb2 = e->prog4c.childs[op.child_begin + 1];
           const int ka = kind4c(ca.kind), kb = kind4c(cb2.kind);
-          if (ka == W4C_TIP && kb == W4C_TIP) shape = W4C_TT;
-          else if (ka == W4C_TIP && kb == W4C_REG) shape = W4C_TS;
-          else if (ka == W4C_REG && kb == W4C_TIP) { shape = W4C_TS; order[0] = 1; order[1] = 0; }
+          const bool wa = ka == W4C_TIP && ca.idx < 0, wb = kb == W4C_TIP && cb2.idx < 0;
+          // a wide tip is consumed first (W4C_WA); two wide tips set both bits
+          if (ka == W4C_TIP && kb == W4C_TIP) {
+            shape = W4C_TT;
+            if (wb && !wa) { order[0] = 1; order[1] = 0; }
+            wide = (wa || wb ? (unsigned)W4C_WA : 0u) | (wa && wb ? (unsigned)W4C_WB : 0u);
+          }
+          else if (ka == W4C_TIP && kb == W4C_REG) { shape = W4C_TS; wide = wa ? (unsigned)W4C_WA : 0u; }
+          else if (ka == W4C_REG && kb == W4C_TIP) { shape = W4C_TS; order[0] = 1; order[1] = 0; wide = wb ? (unsigned)W4C_WA : 0u; }
           else if (ka == W4C_RSL && kb == W4C_REG) shape = W4C_JW;
           else if (ka == W4C_REG && kb == W4C_RSL) { shape = W4C_JW; order[0] = 1; order[1] = 0; }
           else if (ka == W4C_SLOT && kb == W4C_REG) { shape = W4C_JS; jslot = (unsigned)ca.idx; }
           else if (ka == W4C_REG && kb == W4C_SLOT) { shape = W4C_JS; jslot = (unsigned)cb2.idx; order[0] = 1; order[1] = 0; }
         }
-        unsigned d = (unsigned)shape | (op.dst_slot == -2 ? (unsigned)W4C_DSTW : 0u) | ((unsigned)op.nchild << 24);
+        unsigned d = (unsigned)shape | wide | (op.dst_slot == -2 ? (unsigned)W4C_DSTW : 0u) | ((unsigned)op.nchild << 24);
         if (op.dst_slot >= 0) d |= ((unsigned)op.dst_slot << 8) | 0x4000u;
         unsigned d2 = 0;
         int nslot_tok = 0;
@@ -925,17 +958,22 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
             d2 |= (unsigned)kind4c(ch.kind) << (2 * j);
             if (ch.kind == CHILD_SLOT) d2 |= (unsigned)ch.idx << (12 + 6 * nslot_tok++);
           }
+          if (shape == W4C_GENERIC && ch.kind == CHILD_TIP && ch.idx < 0) ok = false;   // (the fathers of cherries are binary)
           Pack4cBlock pb{};
           pb.kind = kind4c(ch.kind);
           pb.pnode = ch.pnode;
+          pb.son0 = pb.son1 = -1;
           pb.off = (long long)((size_t)nchunks * CH + used);
-          e->w4c_blocks.push_back(pb);
-          if (ch.kind == CHILD_TIP) {
-            e->w4c_tip_order.push_back(ch.idx);
-            used += (size_t)blk_tip;
-          } else {
-            used += (size_t)blk_int;
+          if (ch.kind == CHILD_TIP && ch.idx < 0) {
+            pb.kind = W4C_CHERRY;
+            pb.son0 = e->children[e->child_off[ch.pnode]];
+            pb.son1 = e->children[e->child_off[ch.pnode] + 1];
+            e->w4c_tip_order.push_back(make_int2(e->leaf_slot[pb.son0], e->leaf_slot[pb.son1]));
+          } else if (ch.kind == CHILD_TIP) {
+            e->w4c_tip_order.push_back(make_int2(ch.idx, -1));
           }
+          e->w4c_blocks.push_back(pb);
+          used += (size_t)child_bytes(ch);
         }
         if (nslot_tok > 3) ok = false;
         if (nwords < kW4cMaxOps) W.desc[nwords] = make_uint2(d, d2);
@@ -949,6 +987,7 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
       e->w4c_CH = CH;
       e->w4c_stream_bytes = (size_t)nchunks * CH;
       e->w4c = ok;
+      e->w4c_frontier_nodes = ok ? (int)std::count(e->w4c_cherry.begin(), e->w4c_cherry.end(), 1) : 0;
     }
   }
   int rc = upload_program(e, e->prog);
@@ -1095,7 +1134,7 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
     BPP_CUDA(dev_alloc(e, &e->d_w4c_blocks, e->w4c_blocks.size()));
     BPP_CUDA(cudaMemcpy(e->d_w4c_blocks, e->w4c_blocks.data(), e->w4c_blocks.size() * sizeof(Pack4cBlock), cudaMemcpyHostToDevice));
     BPP_CUDA(dev_alloc(e, &e->d_w4c_tip_order, e->w4c_tip_order.size()));
-    BPP_CUDA(cudaMemcpy(e->d_w4c_tip_order, e->w4c_tip_order.data(), e->w4c_tip_order.size() * 4, cudaMemcpyHostToDevice));
+    BPP_CUDA(cudaMemcpy(e->d_w4c_tip_order, e->w4c_tip_order.data(), e->w4c_tip_order.size() * sizeof(int2), cudaMemcpyHostToDevice));
     size_t codes_bytes = 0;
     int parts = 0;
     for (auto& sg : e->w4c_segs) {
@@ -1777,6 +1816,7 @@ static int enqueue_prune(bppgpu_engine* e, int point, int pl, cudaStream_t st) {
     wp.nslots = e->prog4c.nslots;
     wp.ncodes = e->ncodes;
     wp.ntips = (int)e->w4c_tip_order.size();
+    wp.wide_codes = e->ncodes * e->ncodes;
     wp.max_tips = e->w4c_max_tips;
     wp.flags = rflag;
     wp.rootfreq = rootfreq;
@@ -2619,7 +2659,7 @@ static int eval_impl(bppgpu_engine* e, unsigned want, cudaStream_t st, bool time
       if (e->codesT_dirty && e->N > 0) {
         for (const auto& sg : e->w4c_segs) {
           pack_codesC_kernel<<<(unsigned)sg.grid, 256, 0, st>>>(
-              (const unsigned char*)e->d_codes, e->d_w4c_tip_order, (int)e->w4c_tip_order.size(), e->N, sg.pat0, sg.pat_end,
+              (const unsigned char*)e->d_codes, e->d_w4c_tip_order, (int)e->w4c_tip_order.size(), e->ncodes, e->N, sg.pat0, sg.pat_end,
               (e->w4c_nw / C) * 32 * sg.pt, e->d_codesC + sg.codes_off);
           e->stats.kernel_launches++;
         }
@@ -3318,6 +3358,12 @@ int bppgpu_eval_multi(bppgpu_engine* const* engines, int32_t n_engines, unsigned
     if (d1 && (lw & BPPGPU_EVAL_D1)) std::copy(r + 1, r + 1 + nn, d1 + (size_t)p * nn);
     if (d2 && (lw & BPPGPU_EVAL_D2)) std::copy(r + 1 + nn, r + 1 + 2 * nn, d2 + (size_t)p * nn);
   }
+  return BPPGPU_OK;
+}
+
+int bppgpu_get_frontier_nodes(bppgpu_engine* e, int32_t* out) {
+  if (!e || !out) BPP_FAIL(BPPGPU_E_INVALID, "null argument");
+  *out = e->w4c_frontier_nodes;
   return BPPGPU_OK;
 }
 

@@ -123,11 +123,13 @@ struct bppgpu_engine {
   struct W4cSeg { int pt; long long pat0, pat_end; int grid; size_t codes_off; int part0; };
   std::vector<W4cSeg> w4c_segs;
   std::vector<bppgpu::Pack4cBlock> w4c_blocks;
-  std::vector<int> w4c_tip_order;
+  std::vector<int2> w4c_tip_order;          // code rows in consumption order: {leaf slot, -1} or a cherry's {son 0, son 1}
+  std::vector<char> w4c_cherry;            // [nn] node is a folded cherry: a wide tip of prog4c (BPPGPU_W4C_FRONTIER=0: none)
+  int w4c_frontier_nodes = 0;              // folded cherries of the walk4c program in use
   int w4c_CH = 0, w4c_nchunks = 0, w4c_pt = 2, w4c_nw = 8, w4c_max_tips = 16;
   unsigned char* d_w4c_stream = nullptr;   // [pchunk][nchunks][CH]
   bppgpu::Pack4cBlock* d_w4c_blocks = nullptr;
-  int* d_w4c_tip_order = nullptr;
+  int2* d_w4c_tip_order = nullptr;
   unsigned* d_w4c_counter = nullptr;       // CTAs done in the current evaluation (reset by the last one)
   unsigned char* d_codesC = nullptr;       // [grid][ntips][PPC] tip codes as the CTAs stage them
   // CLV storage (one point at a time)

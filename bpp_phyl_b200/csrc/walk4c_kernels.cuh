@@ -30,12 +30,40 @@ constexpr int kW4cStages = 3;
 constexpr int kW4cMaxTipsPerChunk = 16;   // tip-code rows staged with a chunk
 constexpr int kW4cMaxOps = 3072;          // descriptors (8 bytes each) that fit the kernel-parameter block
 constexpr int kW4cMaxChunks = 1024;
+constexpr int kW4cMaxWideCodes = 64;      // code pairs of a folded cherry (ncodes <= 8)
 
-enum W4cKind { W4C_TIP = 0, W4C_SLOT = 1, W4C_REG = 2, W4C_RSL = 3 };
+// W4C_CHERRY only names a table block (Pack4cBlock::kind): the walk reads a cherry as a wide tip
+enum W4cKind { W4C_TIP = 0, W4C_SLOT = 1, W4C_REG = 2, W4C_RSL = 3, W4C_CHERRY = 4 };
 // binary shapes (the only ones a bifurcating tree's planner emits); 0 = generic child loop
-// one-hot shape bits (tested one by one: the dispatch stays a chain of uniform branches)
+// one-hot shape bits (tested one by one: the dispatch stays a chain of uniform branches).  W4C_WA / W4C_WB: the first / second
+// tip block the handler consumes is a wide tip (a folded cherry, below)
 enum W4cShape { W4C_GENERIC = 0, W4C_TS = 1 /* tip + current rows */, W4C_TT = 2, W4C_JW = 4 /* register slot + current rows */,
-                W4C_JS = 8 /* shared-memory slot + current rows */, W4C_DSTW = 16 /* result goes to the register slot */ };
+                W4C_JS = 8 /* shared-memory slot + current rows */, W4C_DSTW = 16 /* result goes to the register slot */,
+                W4C_WA = 32, W4C_WB = 64 };
+
+// Folded cherries.  The conditional likelihood of a cherry (an internal node whose two sons are tips) depends on the pair of
+// tip codes only, so the table pass evaluates it once per code pair -- tip terms, product, rescale, and the father's term
+// P_cherry . l -- and the walk reads the result like a tip: a WIDE TIP with W = ncodes^2 codes (code_a * ncodes + code_b)
+// and an exponent per row.  Block layout: [class][W][4] doubles, then [class][W] int32 exponents.  Every step is the walk's own
+// arithmetic (the functions below are shared by both kernels), so a folded cherry gives the walk's bits.
+__host__ __device__ inline int w4c_wide_block_bytes(int C, int W) { return (C * W * 36 + 15) & ~15; }
+
+// P . l for one row x of P: the association of every tip table and of term_internal
+__device__ __forceinline__ double w4c_dot(double p0, double p1, double p2, double p3, double l0, double l1, double l2, double l3) {
+  return fma(p3, l3, fma(p2, l2, fma(p1, l1, p0 * l0)));
+}
+__device__ __forceinline__ int w4c_max_hi(const double (&a)[4]) {
+  return max(max(hi_word(a[0]), hi_word(a[1])), max(hi_word(a[2]), hi_word(a[3])));
+}
+// the power-of-two rescale of one row whose largest high word is m
+__device__ __forceinline__ void w4c_rescale(double (&a)[4], int m, int& e) {
+  if (m < kScaleThresholdHi && m >= (1 << 20)) {
+    const int k = rescale_shift(m);
+    const double f = pow2(k);
+    a[0] *= f; a[1] *= f; a[2] *= f; a[3] *= f;
+    e += k;
+  }
+}
 
 // The walk program lives in the KERNEL PARAMETER block (constant bank, up to 32 KB since CUDA 12.1): descriptors and chunk
 // records are read with warp-uniform loads and the per-op dispatch runs on the uniform datapath -- no convergence barriers, no
@@ -53,6 +81,7 @@ struct Walk4cParams {
   const unsigned char* stream;       // [nchunks][CH] this point's table chunks
   const unsigned char* codesC;       // [gridDim.x][ntips][PPC] tip codes, consumption order, one byte per pattern
   int nchunks, CH, nslots, ncodes, ntips;
+  int wide_codes;                    // codes of a wide tip (folded cherry): ncodes^2
   int max_tips;                      // tip-code rows a ring stage has room for (the planner never puts more tips in a chunk)
   unsigned flags;                    // bit0: R semantics at the root
   long long pat0, pat_end;           // this launch covers patterns [pat0, pat_end) (a segment of the engine's pattern list)
@@ -109,11 +138,13 @@ struct W4cState {
   unsigned sp;                 // shared address of the next table block of the current chunk (warp-uniform)
   int tip_off;                 // c * ncodes * 32 bytes
   int tip_block;               // C * ncodes * 32 bytes
+  int wide_W;                  // codes of a wide tip (ncodes^2)
   int c;
   unsigned stA, stB, ste;      // shared addresses of the stack planes, already offset by this thread's lane
 
-  __device__ __forceinline__ void term_tip(double (&t)[PT][4]) {
-    const unsigned tb = sp + tip_off;
+  // a tip's rows; a wide tip (wide: warp-uniform) also adds its rows' exponents to e
+  __device__ __forceinline__ void term_tip(double (&t)[PT][4], int (&e)[PT], bool wide) {
+    const unsigned tb = sp + (wide ? (unsigned)(c * wide_W) << 5 : (unsigned)tip_off);
     unsigned code[PT];
 #pragma unroll
     for (int j = 0; j < PT; ++j) code[j] = lds_u8(ca + 32 * j);
@@ -123,8 +154,13 @@ struct W4cState {
       const double2 b = lds128(tb + (code[j] << 5) + 16);
       t[j][0] = a.x; t[j][1] = a.y; t[j][2] = b.x; t[j][3] = b.y;
     }
+    if (wide) {
+      const unsigned te = sp + ((unsigned)(C * wide_W) << 5) + ((unsigned)(c * wide_W) << 2);
+#pragma unroll
+      for (int j = 0; j < PT; ++j) e[j] += lds32(te + (code[j] << 2));
+    }
     ca += PPC;
-    sp += tip_block;
+    sp += wide ? (unsigned)w4c_wide_block_bytes(C, wide_W) : (unsigned)tip_block;
   }
   // t = P . l, l from: the current rows (W4C_REG), the register slot (W4C_RSL) or a shared-memory slot (W4C_SLOT)
   template <int SRC>
@@ -152,7 +188,7 @@ struct W4cState {
       const double2 p01 = lds128(Pm + 32 * x);        // warp-uniform address: broadcast
       const double2 p23 = lds128(Pm + 32 * x + 16);
 #pragma unroll
-      for (int j = 0; j < PT; ++j) t[j][x] = fma(p23.y, l[j][3], fma(p23.x, l[j][2], fma(p01.y, l[j][1], p01.x * l[j][0])));
+      for (int j = 0; j < PT; ++j) t[j][x] = w4c_dot(p01.x, p01.y, p23.x, p23.y, l[j][0], l[j][1], l[j][2], l[j][3]);
     }
   }
   // rescale per row, then store to v (or to the register slot)
@@ -162,19 +198,12 @@ struct W4cState {
     int mmin = 0x7fffffff;
 #pragma unroll
     for (int j = 0; j < PT; ++j) {
-      m[j] = max(max(hi_word(a[j][0]), hi_word(a[j][1])), max(hi_word(a[j][2]), hi_word(a[j][3])));
+      m[j] = w4c_max_hi(a[j]);
       mmin = min(mmin, m[j]);
     }
     if (mmin < kScaleThresholdHi) {  // rare: some row of this thread is small (or identically zero)
 #pragma unroll
-      for (int j = 0; j < PT; ++j) {
-        if (m[j] < kScaleThresholdHi && m[j] >= (1 << 20)) {
-          const int k = rescale_shift(m[j]);
-          const double f = pow2(k);
-          a[j][0] *= f; a[j][1] *= f; a[j][2] *= f; a[j][3] *= f;
-          e[j] += k;
-        }
-      }
+      for (int j = 0; j < PT; ++j) w4c_rescale(a[j], m[j], e[j]);
     }
 #pragma unroll
     for (int j = 0; j < PT; ++j) {
@@ -191,13 +220,13 @@ struct W4cState {
   // join -- are one handler each; the host lays the op's table blocks out in the handler's order (tip block first / the
   // stacked operand's P first).
   template <bool DSTW>
-  __device__ __forceinline__ void op_tt() {
+  __device__ __forceinline__ void op_tt(bool wa, bool wb) {
     double ta[PT][4], tb[PT][4];
     int e[PT];
 #pragma unroll
     for (int j = 0; j < PT; ++j) e[j] = 0;
-    term_tip(ta);
-    term_tip(tb);
+    term_tip(ta, e, wa);
+    term_tip(tb, e, wb);
 #pragma unroll
     for (int j = 0; j < PT; ++j) {
       ta[j][0] *= tb[j][0]; ta[j][1] *= tb[j][1]; ta[j][2] *= tb[j][2]; ta[j][3] *= tb[j][3];
@@ -205,12 +234,12 @@ struct W4cState {
     commit<DSTW>(ta, e);
   }
   template <bool DSTW>
-  __device__ __forceinline__ void op_ts() {
+  __device__ __forceinline__ void op_ts(bool wa) {
     double ta[PT][4], tb[PT][4];
     int e[PT];
 #pragma unroll
     for (int j = 0; j < PT; ++j) e[j] = 0;
-    term_tip(ta);
+    term_tip(ta, e, wa);
     term_internal<W4C_REG>(0, tb, e);
 #pragma unroll
     for (int j = 0; j < PT; ++j) {
@@ -243,7 +272,7 @@ struct W4cState {
     for (int ch = 0; ch < nchild; ++ch, toks >>= 2) {
       const int kind = (int)toks & 3;
       double t[PT][4];
-      if (kind == W4C_TIP) term_tip(t);
+      if (kind == W4C_TIP) term_tip(t, e, false);
       else if (kind == W4C_SLOT) { term_internal<W4C_SLOT>((int)slots & 63, t, e); slots >>= 6; }
       else if (kind == W4C_RSL) term_internal<W4C_RSL>(0, t, e);
       else term_internal<W4C_REG>(0, t, e);
@@ -306,6 +335,7 @@ walk4c_kernel(const __grid_constant__ Walk4cParams prm, const __grid_constant__ 
   s.c = c;
   s.tip_off = c * prm.ncodes * 32;
   s.tip_block = C * prm.ncodes * 32;
+  s.wide_W = prm.wide_codes;
   const unsigned my_code_off = (unsigned)(g * (32 * PT) + lane);
 #pragma unroll
   for (int j = 0; j < PT; ++j) {
@@ -351,15 +381,16 @@ walk4c_kernel(const __grid_constant__ Walk4cParams prm, const __grid_constant__ 
     for (int o = 0; o < n_ops; ++o) {
       const uint2 dd = prog.desc[opi + o];
       const unsigned d = dd.x;
+      const bool wa = d & W4C_WA, wb = d & W4C_WB;
       if (!(d & W4C_DSTW)) {
-        if (d & W4C_TS) s.template op_ts<false>();
-        else if (d & W4C_TT) s.template op_tt<false>();
+        if (d & W4C_TS) s.template op_ts<false>(wa);
+        else if (d & W4C_TT) s.template op_tt<false>(wa, wb);
         else if (d & W4C_JW) s.template op_join<W4C_RSL, false>(0);
         else if (d & W4C_JS) s.template op_join<W4C_SLOT, false>((int)(d >> 16) & 63);
         else s.op_generic((int)(d >> 24) & 0xf, dd.y & 0xfffu, dd.y >> 12, false);
       } else {
-        if (d & W4C_TS) s.template op_ts<true>();
-        else if (d & W4C_TT) s.template op_tt<true>();
+        if (d & W4C_TS) s.template op_ts<true>(wa);
+        else if (d & W4C_TT) s.template op_tt<true>(wa, wb);
         else if (d & W4C_JW) s.template op_join<W4C_RSL, true>(0);
         else if (d & W4C_JS) s.template op_join<W4C_SLOT, true>((int)(d >> 16) & 63);
         else s.op_generic((int)(d >> 24) & 0xf, dd.y & 0xfffu, dd.y >> 12, true);
@@ -454,35 +485,81 @@ walk4c_kernel(const __grid_constant__ Walk4cParams prm, const __grid_constant__ 
 }
 
 // codes [nl][N] (leaf-slot major) -> codesC [cta][tip in consumption order][PPC]: the rows a CTA stages with its chunks
-// (of one segment [pat0, pat_end) of the pattern list, walked by CTAs of PPC patterns)
-__global__ void pack_codesC_kernel(const unsigned char* codes, const int* tip_order, int ntips, long long N, long long pat0,
-                                   long long pat_end, int PPC, unsigned char* codesC) {
+// (of one segment [pat0, pat_end) of the pattern list, walked by CTAs of PPC patterns).  A tip entry is {leaf slot, -1}; a
+// folded cherry's is {leaf slot of son 0, leaf slot of son 1}, whose row is the mixed-radix code code_0 * ncodes + code_1.
+__global__ void pack_codesC_kernel(const unsigned char* codes, const int2* tip_order, int ntips, int ncodes, long long N,
+                                   long long pat0, long long pat_end, int PPC, unsigned char* codesC) {
   const size_t cta = blockIdx.x;
   for (int i = threadIdx.x; i < ntips * PPC; i += blockDim.x) {
     const int k = i / PPC, p = i - k * PPC;
     const long long pat = pat0 + (long long)cta * PPC + p;
-    codesC[(cta * ntips + k) * PPC + p] = pat < pat_end ? codes[(size_t)tip_order[k] * N + pat] : (unsigned char)0;
+    unsigned v = 0;
+    if (pat < pat_end) {
+      const int2 t = tip_order[k];
+      v = codes[(size_t)t.x * N + pat];
+      if (t.y >= 0) v = v * (unsigned)ncodes + codes[(size_t)t.y * N + pat];
+    }
+    codesC[(cta * ntips + k) * PPC + p] = (unsigned char)v;
   }
 }
 
 // table blocks of the chunked stream: one CTA per child block
 struct Pack4cBlock {
-  int kind;       // W4C_TIP or internal
+  int kind;       // W4C_TIP, W4C_CHERRY or internal
   int pnode;      // node whose branch carries the child
+  int son0, son1; // W4C_CHERRY: the cherry's tips, son order
   long long off;  // BYTE offset of the block in the chunked stream
 };
+
+// [class][code][x]: P . (code's tip vector), one tip table
+__device__ __forceinline__ void w4c_tip_block(const double* Pn, const double* code_table, int C, int ncodes, double* out) {
+  for (int e = threadIdx.x; e < ncodes * C * 4; e += blockDim.x) {
+    const int x = e & 3, code = (e >> 2) % ncodes, c = (e >> 2) / ncodes;
+    const double* tv = code_table + code * 4;
+    const double* pr = Pn + c * 16 + x * 4;
+    out[e] = w4c_dot(pr[0], pr[1], pr[2], pr[3], tv[0], tv[1], tv[2], tv[3]);
+  }
+}
+// the wide-tip block of a folded cherry (layout: w4c_wide_block_bytes).  Per (class, code pair) row the steps of the walk's
+// op_tt on the two tips -- tip terms, product, rescale -- and then term_internal of the father's contraction with the
+// cherry's branch P: the row the father would have read, with the exponent it would have added.
+__device__ __forceinline__ void w4c_cherry_block(const double* Pa, const double* Pb, const double* Pn, const double* code_table,
+                                                 int C, int ncodes, unsigned char* out) {
+  const int W = ncodes * ncodes;
+  double* rows = reinterpret_cast<double*>(out);
+  int* exps = reinterpret_cast<int*>(out + (size_t)C * W * 32);
+  for (int r = threadIdx.x; r < C * W; r += blockDim.x) {
+    const int c = r / W, code = r - c * W;
+    const double* ta = code_table + (code / ncodes) * 4;
+    const double* tb = code_table + (code % ncodes) * 4;
+    double a[4];
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      const double* pa = Pa + c * 16 + x * 4;
+      const double* pb = Pb + c * 16 + x * 4;
+      a[x] = w4c_dot(pa[0], pa[1], pa[2], pa[3], ta[0], ta[1], ta[2], ta[3]) *
+             w4c_dot(pb[0], pb[1], pb[2], pb[3], tb[0], tb[1], tb[2], tb[3]);
+    }
+    int e = 0;
+    w4c_rescale(a, w4c_max_hi(a), e);
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      const double* pn = Pn + c * 16 + x * 4;
+      rows[(size_t)r * 4 + x] = w4c_dot(pn[0], pn[1], pn[2], pn[3], a[0], a[1], a[2], a[3]);
+    }
+    exps[r] = e;
+  }
+}
+
 __global__ void pack_stream4c_kernel(const Pack4cBlock* blocks, const double* P /*[nn][C][4][4]*/, const double* code_table,
                                      int C, int ncodes, unsigned char* stream) {
   const Pack4cBlock b = blocks[blockIdx.x];
   const double* Pn = P + (size_t)b.pnode * C * 16;
   double* out = reinterpret_cast<double*>(stream + b.off);
-  if (b.kind == W4C_TIP) {   // [class][code][x]
-    for (int e = threadIdx.x; e < ncodes * C * 4; e += blockDim.x) {
-      const int x = e & 3, code = (e >> 2) % ncodes, c = (e >> 2) / ncodes;
-      const double* tv = code_table + code * 4;
-      const double* pr = Pn + c * 16 + x * 4;
-      out[e] = fma(pr[3], tv[3], fma(pr[2], tv[2], fma(pr[1], tv[1], pr[0] * tv[0])));
-    }
+  if (b.kind == W4C_TIP) {
+    w4c_tip_block(Pn, code_table, C, ncodes, out);
+  } else if (b.kind == W4C_CHERRY) {
+    w4c_cherry_block(P + (size_t)b.son0 * C * 16, P + (size_t)b.son1 * C * 16, Pn, code_table, C, ncodes, stream + b.off);
   } else {                   // [class][x][y] = the reference's pxy_ order
     for (int e = threadIdx.x; e < C * 16; e += blockDim.x) out[e] = Pn[e];
   }
@@ -491,6 +568,7 @@ __global__ void pack_stream4c_kernel(const Pack4cBlock* blocks, const double* P 
 // K1 + K2b fused for the DNA walk (S = 4, real spectra, value only): the CTA of a child block builds the branch's
 // P(t) = V exp(L r_c t) V^-1 for every class -- the arithmetic of pt_eigen_kernel (pt_kernels.cuh), term by term, so the tables are
 // bit-identical -- writes it to the P table (accessors read it there) and lays out its stream block.  One launch instead of two.
+// A cherry block builds the P of its three branches (both tips' and the cherry's own).
 struct PtPack4cParams {
   const Pack4cBlock* blocks;
   const ModelDev* models;
@@ -502,31 +580,36 @@ struct PtPack4cParams {
   double* P;                 // [nn][C][4][4] of this point
   unsigned char* stream;
 };
-__global__ void pt_pack4c_kernel(PtPack4cParams p) {
-  __shared__ double Ps[8 * 16];
-  const Pack4cBlock b = p.blocks[blockIdx.x];
-  const ModelDev md = p.models[p.branch_model[b.pnode]];
+__device__ __forceinline__ void pt4c_branch(const PtPack4cParams& p, int node, double* Ps) {
+  const ModelDev md = p.models[p.branch_model[node]];
   const int C = p.C;
   for (int e = threadIdx.x; e < C * 16; e += blockDim.x) {
     const int c = e >> 4, x = (e >> 2) & 3, y = e & 3;
-    const double l = md.rate * (p.brlen[b.pnode] * p.rates[c]);
+    const double l = md.rate * (p.brlen[node] * p.rates[c]);
     double a0 = 0.0;
 #pragma unroll
     for (int k = 0; k < 4; ++k) a0 = fma(md.V[x * 4 + k] * md.Vinv[k * 4 + y], exp(md.re[k] * l), a0);
     Ps[e] = a0;
-    p.P[(size_t)b.pnode * C * 16 + e] = a0;
+    p.P[(size_t)node * C * 16 + e] = a0;
+  }
+}
+__global__ void pt_pack4c_kernel(PtPack4cParams p) {
+  __shared__ double Ps[3][8 * 16];
+  const Pack4cBlock b = p.blocks[blockIdx.x];
+  const int C = p.C;
+  pt4c_branch(p, b.pnode, Ps[0]);
+  if (b.kind == W4C_CHERRY) {
+    pt4c_branch(p, b.son0, Ps[1]);
+    pt4c_branch(p, b.son1, Ps[2]);
   }
   __syncthreads();
   double* out = reinterpret_cast<double*>(p.stream + b.off);
-  if (b.kind == W4C_TIP) {   // [class][code][x]
-    for (int e = threadIdx.x; e < p.ncodes * C * 4; e += blockDim.x) {
-      const int x = e & 3, code = (e >> 2) % p.ncodes, c = (e >> 2) / p.ncodes;
-      const double* tv = p.code_table + code * 4;
-      const double* pr = Ps + c * 16 + x * 4;
-      out[e] = fma(pr[3], tv[3], fma(pr[2], tv[2], fma(pr[1], tv[1], pr[0] * tv[0])));
-    }
+  if (b.kind == W4C_TIP) {
+    w4c_tip_block(Ps[0], p.code_table, C, p.ncodes, out);
+  } else if (b.kind == W4C_CHERRY) {
+    w4c_cherry_block(Ps[1], Ps[2], Ps[0], p.code_table, C, p.ncodes, p.stream + b.off);
   } else {
-    for (int e = threadIdx.x; e < C * 16; e += blockDim.x) out[e] = Ps[e];
+    for (int e = threadIdx.x; e < C * 16; e += blockDim.x) out[e] = Ps[0][e];
   }
 }
 

@@ -287,6 +287,66 @@ def pt_batch(model: _ModelHolder, t, want=WANT_P, device=0):
     return outs
 
 
+def _device_address(a):
+    """Address of a CUDA tensor or an int address (device memory); None for host arrays."""
+    if isinstance(a, int):
+        return a
+    if hasattr(a, "is_cuda") and a.is_cuda:
+        assert a.is_contiguous()
+        return a.data_ptr()
+    return None
+
+
+def pairwise_distances(codes, weights, code_table, model: _ModelHolder, freqs, rates, probs, device=0, counts=False,
+                       n_leaves=None, n_patterns=None, code_bytes=None):
+    """bppgpu_pairwise_distances: ML distance of every pair of tip-code rows (DistanceEstimation::computeMatrix).
+
+    ``codes``: [L][N] uint8 / uint16 numpy array, or device-resident rows (a contiguous CUDA tensor, or an int address of
+    device memory with ``n_leaves``, ``n_patterns`` and ``code_bytes`` given) such as site_patterns_device writes.
+    ``weights``: [N] (numpy, CUDA tensor or device address).  Returns (dist [L][L], lnl [L][L]) and, with counts=True,
+    also the joint code counts [L(L-1)/2][n_codes][n_codes] of the pairs a < b in row-major upper-triangle order."""
+    table = _f64(code_table)
+    K = table.shape[0]
+    addr = _device_address(codes)
+    if addr is None:
+        c = np.ascontiguousarray(codes)
+        if c.dtype not in (np.uint8, np.uint16):
+            c = np.ascontiguousarray(c, np.uint8 if K <= 256 else np.uint16)
+        L, N = c.shape
+        cb = c.dtype.itemsize
+        cptr, keep_c = c.ctypes.data_as(C.c_void_p), c
+    else:
+        if isinstance(codes, int):
+            L, N, cb = n_leaves, n_patterns, code_bytes
+        else:
+            L, N = codes.shape
+            cb = codes.element_size()
+        cptr, keep_c = C.c_void_p(addr), codes
+    waddr = _device_address(weights)
+    if waddr is None:
+        w = np.ascontiguousarray(weights, np.uint32)
+        wptr = _ptr(w, C.c_uint32)
+    else:
+        w = weights
+        wptr = C.cast(C.c_void_p(waddr), C.POINTER(C.c_uint32))
+    f, r, p = _f64(freqs), _f64(rates), _f64(probs)
+    dist = np.empty((L, L))
+    lnl = np.empty((L, L))
+    cnt = np.empty((L * (L - 1) // 2, K, K), np.uint32) if counts else None
+    _check(lib().bppgpu_pairwise_distances(C.c_int(device), C.byref(model.desc), _ptr(f), C.c_int32(len(r)), _ptr(r), _ptr(p),
+                                           C.c_int32(K), C.c_int32(cb), _ptr(table), C.c_int32(L), C.c_int64(N), cptr, wptr,
+                                           _ptr(dist), _ptr(lnl), _ptr(cnt, C.c_uint32)))
+    del keep_c, w
+    return (dist, lnl, cnt) if counts else (dist, lnl)
+
+
+def pairwise_distances_timing():
+    """Device milliseconds of the last pairwise_distances call on this thread: (upload, counts, ML)."""
+    v = [C.c_double(0) for _ in range(3)]
+    _check(lib().bppgpu_pairwise_distances_timing(*[C.byref(x) for x in v]))
+    return tuple(x.value for x in v)
+
+
 class Engine:
     """Owning wrapper of a ``bppgpu_engine*``."""
 

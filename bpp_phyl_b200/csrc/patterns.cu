@@ -17,6 +17,7 @@
 //   4. tip codes: tip[leaf][pattern] = column[pattern_site[pattern]][leaf] through a shared-memory tile transpose.
 #include "common.cuh"
 #include "bppgpu.h"
+#include "staging.h"
 
 #include <cub/cub.cuh>
 
@@ -30,6 +31,86 @@
 #include <vector>
 
 namespace bppgpu {
+
+// ---- pageable host memory <-> device at PCIe speed (staging.h) -------------------------------------------------------------------
+namespace {
+StagePool g_stage;
+}  // namespace
+
+cudaError_t StagePool::ensure(int dev) {
+  if (device == dev) return cudaSuccess;
+  if (device >= 0) return cudaErrorInvalidDevice;   // one device per process for the pool; other devices take the direct copy
+  const char* e = getenv("BPPGPU_COPY_THREADS");
+  int t = e ? atoi(e) : std::min(4, std::max(1, (int)std::thread::hardware_concurrency()));
+  t = std::max(1, std::min(t, kCopyThreadsMax));
+  for (int i = 0; i < t; ++i) {
+    cudaError_t r = cudaStreamCreateWithFlags(&stream[i], cudaStreamNonBlocking);
+    for (int k = 0; k < 2 && r == cudaSuccess; ++k) {
+      r = cudaHostAlloc(&pinned[i][k], kStageChunk, cudaHostAllocDefault);
+      if (r == cudaSuccess) r = cudaEventCreateWithFlags(&done[i][k], cudaEventDisableTiming);
+    }
+    if (r != cudaSuccess) return r;
+  }
+  threads = t;
+  device = dev;
+  return cudaSuccess;
+}
+
+// blocking copy; the caller has synchronised the work that produced `src` (device to host) / will launch consumers afterwards
+cudaError_t staged_copy(void* dst, const void* src, size_t bytes, bool h2d, int device) {
+  if (bytes == 0) return cudaSuccess;
+  const void* host = h2d ? src : dst;
+  cudaPointerAttributes at;
+  bool pageable = cudaPointerGetAttributes(&at, host) == cudaSuccess && at.type == cudaMemoryTypeUnregistered;
+  cudaGetLastError();
+  std::unique_lock<std::mutex> lock(g_stage.mu, std::defer_lock);
+  if (pageable && bytes >= 4 * kStageChunk) {
+    lock.lock();
+    if (g_stage.ensure(device) != cudaSuccess) { cudaGetLastError(); pageable = false; }
+  } else {
+    pageable = false;
+  }
+  // (cudaMemcpyDefault: the caller's side may also be DEVICE memory -- an alignment already resident, results that stay on the GPU)
+  if (!pageable) return cudaMemcpy(dst, src, bytes, cudaMemcpyDefault);
+  const size_t nchunks = (bytes + kStageChunk - 1) / kStageChunk;
+  const int T = g_stage.threads;
+  std::vector<cudaError_t> err(T, cudaSuccess);
+  auto worker = [&](int t) {
+    cudaError_t r = cudaSetDevice(device);
+    size_t pend_off = 0, pend_len = 0;   // device to host: the chunk whose DMA is in flight, still to be copied out of its slot
+    int pend_slot = -1, it = 0;
+    for (size_t c = (size_t)t; c < nchunks && r == cudaSuccess; c += (size_t)T, ++it) {
+      const int slot = it & 1;
+      const size_t off = c * kStageChunk, len = std::min(kStageChunk, bytes - off);
+      if (h2d) {
+        r = cudaEventSynchronize(g_stage.done[t][slot]);   // the DMA that last read this slot
+        if (r != cudaSuccess) break;
+        std::memcpy(g_stage.pinned[t][slot], (const char*)src + off, len);
+        r = cudaMemcpyAsync((char*)dst + off, g_stage.pinned[t][slot], len, cudaMemcpyHostToDevice, g_stage.stream[t]);
+        if (r == cudaSuccess) r = cudaEventRecord(g_stage.done[t][slot], g_stage.stream[t]);
+      } else {
+        r = cudaMemcpyAsync(g_stage.pinned[t][slot], (const char*)src + off, len, cudaMemcpyDeviceToHost, g_stage.stream[t]);
+        if (r == cudaSuccess) r = cudaEventRecord(g_stage.done[t][slot], g_stage.stream[t]);
+        if (pend_slot >= 0 && r == cudaSuccess) {
+          r = cudaEventSynchronize(g_stage.done[t][pend_slot]);
+          if (r == cudaSuccess) std::memcpy((char*)dst + pend_off, g_stage.pinned[t][pend_slot], pend_len);
+        }
+        pend_slot = slot; pend_off = off; pend_len = len;
+      }
+    }
+    if (r == cudaSuccess) r = cudaStreamSynchronize(g_stage.stream[t]);
+    if (!h2d && pend_slot >= 0 && r == cudaSuccess) std::memcpy((char*)dst + pend_off, g_stage.pinned[t][pend_slot], pend_len);
+    err[t] = r;
+  };
+  std::vector<std::thread> th;
+  for (int t = 1; t < T; ++t) th.emplace_back(worker, t);
+  worker(0);
+  for (auto& x : th) x.join();
+  for (cudaError_t r : err)
+    if (r != cudaSuccess) return r;
+  return cudaSuccess;
+}
+
 namespace {
 
 // key of position i in this pass: bytes [8w, 8w+8) of column perm[i], first byte most significant, zero padded past the end
@@ -112,7 +193,7 @@ __global__ void pattern_tip_codes_kernel(const T* __restrict__ cols, const long 
 
 // ---- "dedup" (the default; BPPGPU_PATTERNS_ALGO=radix selects the plain word-by-word sort of every column) -----------------------
 // Measured on 1M sites x 1024 taxa (245k patterns): the kernels of this variant take 20 ms, the plain sort 57 ms; the rest of a call
-// is the alignment going in and the tip codes coming out (see staged_copy below), against 0.59 s for the host routine
+// is the alignment going in and the tip codes coming out (see staging.h), against 0.59 s for the host routine
 // (profiles/r2_patterns_device_vs_host_1Mx1024.json); outputs identical, bit for bit, in every test.
 // Identical columns are merged BEFORE the lexicographic sort: one 64-bit hash per column (equal columns -> equal hashes; a
 // collision between different columns only leaves duplicates for the final run detection to merge), one stable sort of the hashes,
@@ -204,96 +285,6 @@ struct DevBufs {
   }
   ~DevBufs() { cudaFree(slab); cudaFree(tip); }
 };
-
-// ---- pageable host memory <-> device at PCIe speed ------------------------------------------------------------------------------
-// A plain cudaMemcpy of pageable memory is bounded by ONE host thread copying through the driver's staging buffer (about 10 GB/s);
-// the alignment (1 GB for 1M sites x 1024 taxa) and the tip codes coming back are most of this routine's time.  Here kCopyThreads
-// host threads each move their share of the 4 MB chunks through two pinned buffers of their own, on their own stream, so that the
-// host-side memcpy of one chunk overlaps the DMA of the others.  The pinned pool is allocated once per process.  Buffers the
-// runtime already knows (pinned / registered / device / managed) and small ones take the direct copy.
-constexpr size_t kStageChunk = (size_t)4 << 20;
-constexpr int kCopyThreadsMax = 8;
-struct StagePool {
-  std::mutex mu;
-  int device = -1, threads = 0;
-  void* pinned[kCopyThreadsMax][2] = {};
-  cudaStream_t stream[kCopyThreadsMax] = {};
-  cudaEvent_t done[kCopyThreadsMax][2] = {};
-  cudaError_t ensure(int dev) {
-    if (device == dev) return cudaSuccess;
-    if (device >= 0) return cudaErrorInvalidDevice;   // one device per process for the pool; other devices take the direct copy
-    const char* e = getenv("BPPGPU_COPY_THREADS");
-    int t = e ? atoi(e) : std::min(4, std::max(1, (int)std::thread::hardware_concurrency()));
-    t = std::max(1, std::min(t, kCopyThreadsMax));
-    for (int i = 0; i < t; ++i) {
-      cudaError_t r = cudaStreamCreateWithFlags(&stream[i], cudaStreamNonBlocking);
-      for (int k = 0; k < 2 && r == cudaSuccess; ++k) {
-        r = cudaHostAlloc(&pinned[i][k], kStageChunk, cudaHostAllocDefault);
-        if (r == cudaSuccess) r = cudaEventCreateWithFlags(&done[i][k], cudaEventDisableTiming);
-      }
-      if (r != cudaSuccess) return r;
-    }
-    threads = t;
-    device = dev;
-    return cudaSuccess;
-  }
-};
-StagePool g_stage;
-
-// blocking copy; the caller has synchronised the work that produced `src` (device to host) / will launch consumers afterwards
-cudaError_t staged_copy(void* dst, const void* src, size_t bytes, bool h2d, int device) {
-  if (bytes == 0) return cudaSuccess;
-  const void* host = h2d ? src : dst;
-  cudaPointerAttributes at;
-  bool pageable = cudaPointerGetAttributes(&at, host) == cudaSuccess && at.type == cudaMemoryTypeUnregistered;
-  cudaGetLastError();
-  std::unique_lock<std::mutex> lock(g_stage.mu, std::defer_lock);
-  if (pageable && bytes >= 4 * kStageChunk) {
-    lock.lock();
-    if (g_stage.ensure(device) != cudaSuccess) { cudaGetLastError(); pageable = false; }
-  } else {
-    pageable = false;
-  }
-  // (cudaMemcpyDefault: the caller's side may also be DEVICE memory -- an alignment already resident, results that stay on the GPU)
-  if (!pageable) return cudaMemcpy(dst, src, bytes, cudaMemcpyDefault);
-  const size_t nchunks = (bytes + kStageChunk - 1) / kStageChunk;
-  const int T = g_stage.threads;
-  std::vector<cudaError_t> err(T, cudaSuccess);
-  auto worker = [&](int t) {
-    cudaError_t r = cudaSetDevice(device);
-    size_t pend_off = 0, pend_len = 0;   // device to host: the chunk whose DMA is in flight, still to be copied out of its slot
-    int pend_slot = -1, it = 0;
-    for (size_t c = (size_t)t; c < nchunks && r == cudaSuccess; c += (size_t)T, ++it) {
-      const int slot = it & 1;
-      const size_t off = c * kStageChunk, len = std::min(kStageChunk, bytes - off);
-      if (h2d) {
-        r = cudaEventSynchronize(g_stage.done[t][slot]);   // the DMA that last read this slot
-        if (r != cudaSuccess) break;
-        std::memcpy(g_stage.pinned[t][slot], (const char*)src + off, len);
-        r = cudaMemcpyAsync((char*)dst + off, g_stage.pinned[t][slot], len, cudaMemcpyHostToDevice, g_stage.stream[t]);
-        if (r == cudaSuccess) r = cudaEventRecord(g_stage.done[t][slot], g_stage.stream[t]);
-      } else {
-        r = cudaMemcpyAsync(g_stage.pinned[t][slot], (const char*)src + off, len, cudaMemcpyDeviceToHost, g_stage.stream[t]);
-        if (r == cudaSuccess) r = cudaEventRecord(g_stage.done[t][slot], g_stage.stream[t]);
-        if (pend_slot >= 0 && r == cudaSuccess) {
-          r = cudaEventSynchronize(g_stage.done[t][pend_slot]);
-          if (r == cudaSuccess) std::memcpy((char*)dst + pend_off, g_stage.pinned[t][pend_slot], pend_len);
-        }
-        pend_slot = slot; pend_off = off; pend_len = len;
-      }
-    }
-    if (r == cudaSuccess) r = cudaStreamSynchronize(g_stage.stream[t]);
-    if (!h2d && pend_slot >= 0 && r == cudaSuccess) std::memcpy((char*)dst + pend_off, g_stage.pinned[t][pend_slot], pend_len);
-    err[t] = r;
-  };
-  std::vector<std::thread> th;
-  for (int t = 1; t < T; ++t) th.emplace_back(worker, t);
-  worker(0);
-  for (auto& x : th) x.join();
-  for (cudaError_t r : err)
-    if (r != cudaSuccess) return r;
-  return cudaSuccess;
-}
 
 // BPPGPU_PATTERNS_TRACE=1: stage times on stderr (each stage synchronised; for profiling, not for timing a production call)
 struct StageTrace {

@@ -10,6 +10,7 @@
 //   Model/RateDistribution/{Constant,GammaDiscrete}RateDistribution.h          same names
 //   TreeTemplate.h / TreeTemplateTools (parenthesisToTree, unroot, getNodes)   TreeTemplate<Node>, TreeTemplateTools
 //   SitePatterns.cpp:52-106                                                    SitePatterns (via bppgpu_site_patterns)
+//   Distance/{DistanceMatrix.h,DistanceEstimation,BioNJ}.cpp                   same names (distances on the device, BIONJ on the host)
 //   Likelihood/{R,DR}HomogeneousTreeLikelihood, DRNonHomogeneousTreeLikelihood same names; computeTreeLikelihood,
 //       fireParameterChanged, getValue, get{First,Second}OrderDerivative ... run on the device through libbppgpu
 //
@@ -20,5 +21,7 @@
 #pragma once
 // The classes live in shim/: core.hpp (bpp-core stand-ins, host linear algebra) <- seq.hpp (alphabets, containers) <- tree.hpp
 // <- io.hpp (Newick, Fasta, Phylip, chrFasta readers) <- models.hpp (rate distributions, substitution models, model sets) <- likelihood.hpp (SitePatterns, tree likelihoods)
-// <- ancestral.hpp (reconstruction classes) <- optimizers.hpp (batched Brent, ChromosomeNumberOptimizer, PseudoNewtonOptimizer).
+// <- ancestral.hpp (reconstruction classes) <- optimizers.hpp (batched Brent, ChromosomeNumberOptimizer, PseudoNewtonOptimizer);
+// likelihood.hpp <- distance.hpp (DistanceMatrix, DistanceEstimation, BioNJ).
 #include "shim/optimizers.hpp"
+#include "shim/distance.hpp"

@@ -36,6 +36,43 @@ class SitePatterns {
   std::vector<unsigned int> weights_;
 };
 
+// ---- sites -> patterns -> tip codes ------------------------------------------------------------------------------------------------
+// What the engine and the distance routine consume: the global pattern compression of the sequences `names` (in that order), one
+// code row per sequence (code = index of the distinct character, in order of first appearance) and the code table
+// table[code][state] = model.getInitValue(state, character).
+struct TipCodes {
+  std::vector<unsigned int> weights;            // [patterns]
+  std::vector<int64_t> siteIndex;               // [sites] -> pattern
+  std::vector<std::vector<uint16_t> > codes;    // [names][patterns]
+  std::vector<double> table;                    // [nCodes][S]
+  size_t nCodes;
+};
+inline TipCodes encodeTipCodes(const VectorSiteContainer& sites, const std::vector<std::string>& names, const SubstitutionModel& model) {
+  SitePatterns patterns(sites, names);
+  TipCodes tc;
+  const size_t np = patterns.getWeights().size();
+  tc.weights = patterns.getWeights();
+  tc.siteIndex = patterns.getIndices();
+  std::map<std::string, int> codeOf;
+  std::vector<std::string> chars;
+  tc.codes.assign(names.size(), std::vector<uint16_t>(np));
+  for (size_t t = 0; t < names.size(); ++t) {
+    const BasicSequence& seq = sites.getSequence(names[t]);
+    for (size_t k = 0; k < np; ++k) {
+      const std::string& ch = seq[(size_t)patterns.getPatternSites()[k]];
+      std::map<std::string, int>::iterator it = codeOf.find(ch);
+      if (it == codeOf.end()) { it = codeOf.insert(std::make_pair(ch, (int)chars.size())).first; chars.push_back(ch); }
+      tc.codes[t][k] = (uint16_t)it->second;
+    }
+  }
+  const size_t S = model.getNumberOfStates();
+  tc.nCodes = chars.size();
+  tc.table.resize(chars.size() * S);
+  for (size_t k = 0; k < chars.size(); ++k)
+    for (size_t s = 0; s < S; ++s) tc.table[k * S + s] = model.getInitValue(s, chars[k]);
+  return tc;
+}
+
 // ---- tree likelihood ---------------------------------------------------------------------------------------------------------------
 struct Parameter {
   std::string name;
@@ -362,26 +399,12 @@ class AbstractHomogeneousTreeLikelihood {
     if (sites.getNumberOfSequences() == 0 || sites.getNumberOfSites() == 0)
       throw Exception("DRASRTreeLikelihoodData::initLikelihoods. Can't use empty dataset (0 sequences or 0 sites).");
     const std::vector<std::string> leafNames = tree_->getLeavesNames();
-    SitePatterns patterns(sites, leafNames);
-    nPatterns_ = (int64_t)patterns.getWeights().size();
-    siteIndex_ = patterns.getIndices();
-    // distinct characters -> code table rows (getInitValue)
-    std::map<std::string, int> codeOf;
-    std::vector<std::string> chars;
-    std::vector<std::vector<uint16_t> > codes(leafNames.size(), std::vector<uint16_t>((size_t)nPatterns_));
-    for (size_t t = 0; t < leafNames.size(); ++t) {
-      const BasicSequence& seq = sites.getSequence(leafNames[t]);
-      for (int64_t k = 0; k < nPatterns_; ++k) {
-        const std::string& ch = seq[(size_t)patterns.getPatternSites()[(size_t)k]];
-        std::map<std::string, int>::iterator it = codeOf.find(ch);
-        if (it == codeOf.end()) { it = codeOf.insert(std::make_pair(ch, (int)chars.size())).first; chars.push_back(ch); }
-        codes[t][(size_t)k] = (uint16_t)it->second;
-      }
-    }
+    const TipCodes tc = encodeTipCodes(sites, leafNames, *model_);
+    nPatterns_ = (int64_t)tc.weights.size();
+    siteIndex_ = tc.siteIndex;
+    const std::vector<std::vector<uint16_t> >& codes = tc.codes;
+    const std::vector<double>& table = tc.table;
     const size_t S = model_->getNumberOfStates(), C = rDist_->getNumberOfCategories();
-    std::vector<double> table(chars.size() * S);
-    for (size_t k = 0; k < chars.size(); ++k)
-      for (size_t s = 0; s < S; ++s) table[k * S + s] = model_->getInitValue(s, chars[k]);
     // flattened topology: node id = post-order position
     const int nn = (int)nodes_.size();
     std::vector<int32_t> off(nn + 1, 0), children;
@@ -394,7 +417,7 @@ class AbstractHomogeneousTreeLikelihood {
     cfg.n_states = (int32_t)S; cfg.n_cats = (int32_t)C; cfg.n_patterns = nPatterns_; cfg.n_nodes = nn; cfg.root = nn - 1;
     cfg.child_offsets = off.data(); cfg.children = children.data(); cfg.n_points = nPoints_;
     cfg.n_models = modelSet_ ? (int32_t)modelSet_->getNumberOfModels() : (nModelSlots_ > 0 ? nModelSlots_ : nPoints_);
-    cfg.n_codes = (int32_t)chars.size(); cfg.code_bytes = chars.size() > 256 ? 2 : 1; cfg.code_table = table.data();
+    cfg.n_codes = (int32_t)tc.nCodes; cfg.code_bytes = tc.nCodes > 256 ? 2 : 1; cfg.code_table = table.data();
     // a batch of parameter points on one character keeps no per-node arrays: the engine may then apply P(t) in factored form
     cfg.device = device_; cfg.flags = engineFlags_ | ((nPoints_ > 1 && nPatterns_ == 1 && C == 1) ? 0u : (unsigned)BPPGPU_FLAG_KEEP_CLVS);
     if (engine_) { bppgpu_destroy(engine_); engine_ = nullptr; }
@@ -408,8 +431,8 @@ class AbstractHomogeneousTreeLikelihood {
         check(bppgpu_set_tip_codes(engine_, leaves[t]->getId(), codes[t].data()), "setData");
       }
     }
-    check(bppgpu_set_pattern_weights(engine_, patterns.getWeights().data()), "setData");
-    patternWeights_ = patterns.getWeights();
+    check(bppgpu_set_pattern_weights(engine_, tc.weights.data()), "setData");
+    patternWeights_ = tc.weights;
     hasData_ = true;
     uploadModel();
   }

@@ -127,6 +127,25 @@ enum { BPPGPU_WANT_P = 1, BPPGPU_WANT_DP = 2, BPPGPU_WANT_D2P = 4 };
 int bppgpu_pt_batch(int device, const bppgpu_model_desc* model, int64_t n_t, const double* t,
                     unsigned want, double* P, double* dP, double* d2P);
 
+/* ---- pairwise distances (no tree needed) ------------------------------------
+ * DistanceEstimation::computeMatrix (Distance/DistanceEstimation.cpp) with TwoTreeLikelihood per pair: ML distance of every
+ * pair of the L tip-code rows under one model + rate classes (semantics in DESIGN §7b).  tip_codes [L][N] (elements of
+ * code_bytes = 1 or 2 bytes, as bppgpu_site_patterns_device writes them), weights [N]: host, pinned or device memory of
+ * `device`.  code_table [n_codes][S] as in bppgpu_config, n_codes <= 128; freqs [S] = the model's frequencies (the pair is
+ * rooted at its first sequence).  dist [L][L]: the maximiser of lnL_ab(t) over [1e-6, 1e4] (a bound exactly when the optimum
+ * is there; 1e-6 for a pair every site of which involves a fully ambiguous code; diagonal 0).  lnl [L][L] (value at the
+ * optimum, row sequence as the root side; diagonal 0) and counts [L(L-1)/2][n_codes][n_codes] (joint code counts of the
+ * pairs a < b, row-major upper triangle) may be NULL.  BPPGPU_E_INVALID for a model that is not diagonalizable and
+ * non-singular with a real spectrum (or has the chromosome P(t) semantics), L < 2, a code >= n_codes, or a total weight
+ * >= 2^31.                                                                                                                 */
+int bppgpu_pairwise_distances(int device, const bppgpu_model_desc* model, const double* freqs, int32_t n_cats,
+                              const double* rates, const double* probs, int32_t n_codes, int32_t code_bytes,
+                              const double* code_table, int32_t n_leaves, int64_t n_patterns, const void* tip_codes,
+                              const uint32_t* weights, double* dist, double* lnl, uint32_t* counts);
+/* device time of the calling thread's last successful bppgpu_pairwise_distances, by phase (CUDA events): upload (weights,
+ * tip codes in, packing), pair counts, ML search; summed over the pair blocks; any pointer may be NULL                      */
+int bppgpu_pairwise_distances_timing(double* upload_ms, double* count_ms, double* ml_ms);
+
 /* ---- Interface 2: tree likelihood engine ----------------------------------- */
 typedef struct bppgpu_engine bppgpu_engine;
 

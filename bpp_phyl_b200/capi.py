@@ -347,6 +347,91 @@ def pairwise_distances_timing():
     return tuple(x.value for x in v)
 
 
+class Parsimony:
+    """Owning wrapper of a ``bppgpu_parsimony*``: Fitch parsimony over resident tip sets, topology per call.
+
+    ``codes``: [L][N] uint8 / uint16 numpy array, or device-resident rows (a contiguous CUDA tensor, or an int address of
+    device memory with ``n_leaves``, ``n_patterns`` and ``code_bytes`` given).  ``weights``: [N] (numpy, CUDA tensor or
+    device address).  ``code_table`` [n_codes][n_states]: the set of a code has bit x iff its entry x is > 0.  ``max_bytes``
+    caps the per-pattern-block device arrays (0 = the library's default)."""
+
+    def __init__(self, code_table, codes, weights, device=0, max_bytes=0, n_leaves=None, n_patterns=None, code_bytes=None):
+        self._h = C.c_void_p()
+        table = _f64(code_table)
+        K, S = table.shape
+        addr = _device_address(codes)
+        if addr is None:
+            c = np.ascontiguousarray(codes)
+            if c.dtype not in (np.uint8, np.uint16):
+                c = np.ascontiguousarray(c, np.uint8 if K <= 256 else np.uint16)
+            L, N = c.shape
+            cb = c.dtype.itemsize
+            cptr = c.ctypes.data_as(C.c_void_p)
+        else:
+            if isinstance(codes, int):
+                L, N, cb = n_leaves, n_patterns, code_bytes
+            else:
+                L, N = codes.shape
+                cb = codes.element_size()
+            c, cptr = codes, C.c_void_p(addr)
+        waddr = _device_address(weights)
+        if waddr is None:
+            w = np.ascontiguousarray(weights, np.uint32)
+            wptr = _ptr(w, C.c_uint32)
+        else:
+            w, wptr = weights, C.cast(C.c_void_p(waddr), C.POINTER(C.c_uint32))
+        self.n_leaves, self.N = L, N
+        _check(lib().bppgpu_parsimony_create(C.c_int(device), C.c_int32(S), C.c_int32(K), C.c_int32(cb), _ptr(table),
+                                             C.c_int32(L), C.c_int64(N), cptr, wptr, C.c_int64(max_bytes), C.byref(self._h)))
+        del c, w
+
+    @staticmethod
+    def _topology(child_offsets, children, leaf_row):
+        off = np.ascontiguousarray(child_offsets, np.int32)
+        ch = np.ascontiguousarray(children, np.int32)
+        lr = np.ascontiguousarray(leaf_row, np.int32)
+        return len(off) - 1, (off, ch, lr), (_ptr(off, C.c_int32), _ptr(ch, C.c_int32), _ptr(lr, C.c_int32))
+
+    def score(self, child_offsets, children, root, leaf_row, site_scores=False):
+        """bppgpu_parsimony_score: the weighted score (int), and with site_scores=True also the per-pattern scores [N] uint32."""
+        n, keep, ptrs = self._topology(child_offsets, children, leaf_row)
+        s = C.c_int64(0)
+        sc = np.empty(self.N, np.uint32) if site_scores else None
+        _check(lib().bppgpu_parsimony_score(self._h, C.c_int32(n), C.c_int32(root), *ptrs, C.byref(s), _ptr(sc, C.c_uint32)))
+        return (s.value, sc) if site_scores else s.value
+
+    def nni_deltas(self, child_offsets, children, root, leaf_row):
+        """bppgpu_parsimony_nni: (delta [n_nodes] int64 = new - current score of each node's NNI, 0 where none; score)."""
+        n, keep, ptrs = self._topology(child_offsets, children, leaf_row)
+        d = np.zeros(n, np.int64)
+        s = C.c_int64(0)
+        _check(lib().bppgpu_parsimony_nni(self._h, C.c_int32(n), C.c_int32(root), *ptrs, _ptr(d, C.c_int64), C.byref(s)))
+        return d, s.value
+
+    def last_ms(self):
+        """Device milliseconds of the passes of the last score / nni_deltas call."""
+        ms = C.c_double(0)
+        _check(lib().bppgpu_parsimony_last_ms(self._h, C.byref(ms)))
+        return ms.value
+
+    def close(self):
+        if self._h:
+            lib().bppgpu_parsimony_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+
 class Engine:
     """Owning wrapper of a ``bppgpu_engine*``."""
 

@@ -11,6 +11,7 @@
 //   TreeTemplate.h / TreeTemplateTools (parenthesisToTree, unroot, getNodes)   TreeTemplate<Node>, TreeTemplateTools
 //   SitePatterns.cpp:52-106                                                    SitePatterns (via bppgpu_site_patterns)
 //   Distance/{DistanceMatrix.h,DistanceEstimation,BioNJ}.cpp                   same names (distances on the device, BIONJ on the host)
+//   Parsimony/DRTreeParsimonyScore.cpp, OptimizationTools::optimizeTreeNNI     same names (scores and NNI changes on the device)
 //   Likelihood/{R,DR}HomogeneousTreeLikelihood, DRNonHomogeneousTreeLikelihood same names; computeTreeLikelihood,
 //       fireParameterChanged, getValue, get{First,Second}OrderDerivative ... run on the device through libbppgpu
 //
@@ -22,6 +23,8 @@
 // The classes live in shim/: core.hpp (bpp-core stand-ins, host linear algebra) <- seq.hpp (alphabets, containers) <- tree.hpp
 // <- io.hpp (Newick, Fasta, Phylip, chrFasta readers) <- models.hpp (rate distributions, substitution models, model sets) <- likelihood.hpp (SitePatterns, tree likelihoods)
 // <- ancestral.hpp (reconstruction classes) <- optimizers.hpp (batched Brent, ChromosomeNumberOptimizer, PseudoNewtonOptimizer);
-// likelihood.hpp <- distance.hpp (DistanceMatrix, DistanceEstimation, BioNJ).
+// likelihood.hpp <- distance.hpp (DistanceMatrix, DistanceEstimation, BioNJ); likelihood.hpp <- parsimony.hpp (DRTreeParsimonyScore,
+// OptimizationTools::optimizeTreeNNI).
 #include "shim/optimizers.hpp"
 #include "shim/distance.hpp"
+#include "shim/parsimony.hpp"

@@ -1,5 +1,7 @@
 // bppgpu shim (see ../bppgpu_shim.hpp): SitePatterns and the tree-likelihood classes (R / DR / NH / clock / point batch / mixtures)
 #pragma once
+#include <functional>
+
 #include "models.hpp"
 
 namespace bppshim {
@@ -39,7 +41,7 @@ class SitePatterns {
 // ---- sites -> patterns -> tip codes ------------------------------------------------------------------------------------------------
 // What the engine and the distance routine consume: the global pattern compression of the sequences `names` (in that order), one
 // code row per sequence (code = index of the distinct character, in order of first appearance) and the code table
-// table[code][state] = model.getInitValue(state, character).
+// table[code][state] = initValue(state, character) (the model's getInitValue for the likelihood classes and distances).
 struct TipCodes {
   std::vector<unsigned int> weights;            // [patterns]
   std::vector<int64_t> siteIndex;               // [sites] -> pattern
@@ -47,7 +49,8 @@ struct TipCodes {
   std::vector<double> table;                    // [nCodes][S]
   size_t nCodes;
 };
-inline TipCodes encodeTipCodes(const VectorSiteContainer& sites, const std::vector<std::string>& names, const SubstitutionModel& model) {
+inline TipCodes encodeTipCodes(const VectorSiteContainer& sites, const std::vector<std::string>& names, size_t S,
+                               const std::function<double(size_t, const std::string&)>& initValue) {
   SitePatterns patterns(sites, names);
   TipCodes tc;
   const size_t np = patterns.getWeights().size();
@@ -65,12 +68,15 @@ inline TipCodes encodeTipCodes(const VectorSiteContainer& sites, const std::vect
       tc.codes[t][k] = (uint16_t)it->second;
     }
   }
-  const size_t S = model.getNumberOfStates();
   tc.nCodes = chars.size();
   tc.table.resize(chars.size() * S);
   for (size_t k = 0; k < chars.size(); ++k)
-    for (size_t s = 0; s < S; ++s) tc.table[k * S + s] = model.getInitValue(s, chars[k]);
+    for (size_t s = 0; s < S; ++s) tc.table[k * S + s] = initValue(s, chars[k]);
   return tc;
+}
+inline TipCodes encodeTipCodes(const VectorSiteContainer& sites, const std::vector<std::string>& names, const SubstitutionModel& model) {
+  return encodeTipCodes(sites, names, model.getNumberOfStates(),
+                        [&model](size_t s, const std::string& ch) { return model.getInitValue(s, ch); });
 }
 
 // ---- tree likelihood ---------------------------------------------------------------------------------------------------------------

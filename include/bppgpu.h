@@ -146,6 +146,36 @@ int bppgpu_pairwise_distances(int device, const bppgpu_model_desc* model, const 
  * tip codes in, packing), pair counts, ML search; summed over the pair blocks; any pointer may be NULL                      */
 int bppgpu_pairwise_distances_timing(double* upload_ms, double* count_ms, double* ml_ms);
 
+/* ---- Fitch parsimony (no model; topology per call) ---------------------------
+ * Parsimony/DRTreeParsimonyScore.cpp: computeScoresFromArrays (score, per-site scores) and testNNI (the change of score of
+ * every nearest-neighbour interchange), Fitch's rule on bitsets with double-recursive arrays; semantics in DESIGN §7b.
+ * The handle holds the tip sets resident; the topology is passed to every call, because an NNI search changes it every round.
+ *
+ * bppgpu_parsimony_create (the DRTreeParsimonyScore constructor's data part): tip_codes [n_leaves][n_patterns] (elements of
+ * code_bytes = 1 or 2 bytes; host, pinned or device memory of `device`), weights [n_patterns] (SitePatterns::getWeights).
+ * code_table [n_codes][n_states] as in bppgpu_config: the Fitch set of a code has bit x iff code_table[code][x] > 0.
+ * max_bytes caps the device bytes of the per-pattern-block arrays (0 = default 8 GB).  BPPGPU_E_INVALID for n_states > 32,
+ * a code row with no positive entry, more than 8192 codes, or a tip code >= n_codes.                                       */
+typedef struct bppgpu_parsimony bppgpu_parsimony;
+int bppgpu_parsimony_create(int device, int32_t n_states, int32_t n_codes, int32_t code_bytes, const double* code_table,
+                            int32_t n_leaves, int64_t n_patterns, const void* tip_codes, const uint32_t* weights,
+                            int64_t max_bytes, bppgpu_parsimony** out);
+/* DRTreeParsimonyScore::getScore / getScoreForEachSite for a topology: CSR child_offsets [n_nodes + 1], children, root, and
+ * leaf_row [n_nodes] = tip row of each leaf (ignored for internal nodes).  Sons are merged in son order (the reference's rule
+ * at multifurcations).  score = sum_i w_i c_i (int64); site_scores [n_patterns] = c_i, may be NULL.  BPPGPU_E_INVALID unless
+ * every node is reached exactly once from the root, the root has sons, and every leaf names a distinct row in range.       */
+int bppgpu_parsimony_score(bppgpu_parsimony* h, int32_t n_nodes, int32_t root, const int32_t* child_offsets,
+                           const int32_t* children, const int32_t* leaf_row, int64_t* score, uint32_t* site_scores);
+/* DRTreeParsimonyScore::testNNI for every node at once: delta [n_nodes] = new score - current score of the NNI that swaps v
+ * with its uncle g.son(pos > 1 ? 0 : 1 - pos) (f = father of v, g = father of f, pos = position of f among g's sons); 0 for
+ * nodes without one (the root and its sons).  score (may be NULL) = the current score.  Needs a binary topology with a
+ * three-son root (BPPGPU_E_INVALID otherwise).                                                                               */
+int bppgpu_parsimony_nni(bppgpu_parsimony* h, int32_t n_nodes, int32_t root, const int32_t* child_offsets,
+                         const int32_t* children, const int32_t* leaf_row, int64_t* delta, int64_t* score);
+/* device time (CUDA events) of the passes of the handle's last successful score / nni call */
+int bppgpu_parsimony_last_ms(bppgpu_parsimony* h, double* ms);
+int bppgpu_parsimony_destroy(bppgpu_parsimony* h);
+
 /* ---- Interface 2: tree likelihood engine ----------------------------------- */
 typedef struct bppgpu_engine bppgpu_engine;
 

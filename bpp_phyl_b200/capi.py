@@ -615,4 +615,6 @@ class Engine:
         nf = C.c_int32(0)
         _check(lib().bppgpu_get_frontier_nodes(self._h, C.byref(nf)))
         out["w4c_frontier_nodes"] = nf.value
+        _check(lib().bppgpu_get_three_tip_nodes(self._h, C.byref(nf)))
+        out["w4c_three_tip_nodes"] = nf.value
         return out

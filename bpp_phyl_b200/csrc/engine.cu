@@ -88,7 +88,8 @@ static int ilog2(int v) {
 // op stays the reference's son order (RHomogeneousTreeLikelihood.cpp:827-861).
 // reg_slot (walk4c): a push whose lifetime contains no other push -- the sibling evaluated next has label 1, i.e. is a
 // caterpillar -- goes to the kernel's register slot (dst_slot = -2, child kind CHILD_RSLOT) instead of a shared-memory slot.
-// folded (walk4c): nodes the program treats as tips (CHILD_TIP, idx -1): cherries whose rows the table pass computes.
+// folded (walk4c): nodes the program treats as tips (CHILD_TIP, idx -1): cherries and three-tip subtrees whose rows the
+// table pass computes.
 static void build_program(bppgpu_engine* e, Program& pr, bool all_keep, bool reg_slot = false,
                           const std::vector<char>* folded = nullptr) {
   const int nn = e->nn;
@@ -634,7 +635,7 @@ int bppgpu_destroy(bppgpu_engine* e) {
                   e->d_d2P, e->d_tiptab, e->d_keep, e->d_keep_exp, e->d_gstack, e->d_gstack_exp, e->d_upper,
                   e->d_upper_exp, e->d_SR, e->d_rexp, e->d_site_lnl, e->d_partials, e->d_partials2, e->d_out,
                   e->prog.d_ops, e->prog.d_childs, e->gprog.d_ops, e->gprog.d_childs, e->d_sibs, e->d_scratch,
-                  e->d_dtiptab, e->d_d2tiptab, e->d_dLc, e->d_fam_mask, e->d_fam_part, e->d_fam_packA, e->d_fam_packS, e->d_fam_packL, e->d_fam_packT, e->d_w4c_stream, e->d_w4c_blocks, e->d_w4c_tip_order, e->d_codesC, e->d_w4c_counter, e->d_w4_desc, e->d_w4_tip_order, e->d_w4_blocks, e->d_w4_stream, e->d_codesT,
+                  e->d_dtiptab, e->d_d2tiptab, e->d_dLc, e->d_fam_mask, e->d_fam_part, e->d_fam_packA, e->d_fam_packS, e->d_fam_packL, e->d_fam_packT, e->d_w4c_stream, e->d_w4c_blocks, e->d_w4c_tip_order, e->d_codesC, e->d_w4c_counter, e->d_w4c_block_counter, e->d_w4c_csum, e->d_w4c_cexp, e->d_w4_desc, e->d_w4_tip_order, e->d_w4_blocks, e->d_w4_stream, e->d_codesT,
                   e->d_status, e->d_wr_recs, e->d_chr_tile_edges, e->d_chr_tile_kind, e->d_chr_leaf_state, e->d_child_off,
                   e->d_children, e->d_chr_leaf_vec, e->d_chr_term, e->d_chr_term_exp, e->d_chr_bad, e->d_chr_guardP, e->d_chr_aslab, e->d_prune_nodes, e->d_family_nodes, e->d_chr_probe_t,
                   e->d_chr_probe_bm, e->d_models_noclamp, e->d_bad_idx, e->d_bad_brlen, e->d_bad_rootfreq, e->d_bad_rootfreq_used,
@@ -788,35 +789,95 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
   }
   if (e->path == PATH_WALK4 && !e->keep && !(getenv("BPPGPU_WALK4C") && atoi(getenv("BPPGPU_WALK4C")) == 0)) {
     // walk4c: the same walk with leaf pushes in the register slot, tables cut into fixed-size chunks in walk order, the
-    // program (descriptor words + chunk records) in the kernel-parameter block
-    const int W = e->ncodes * e->ncodes;
-    const int blk_int = C * 128, blk_tip = C * e->ncodes * 32, blk_wide = w4c_wide_block_bytes(C, W);
-    // chunk geometry: bytes of tables and tip-code rows per ring stage (tuning knobs; a stage must hold the largest op)
-    int CH = getenv("BPPGPU_WALK4_CH") ? std::max(1024, atoi(getenv("BPPGPU_WALK4_CH")) & ~127) : 8192;
-    // Folded cherries: a cherry whose father is binary becomes a wide tip of the father (walk4c_kernels.cuh), its op leaves
-    // the walk.  W <= 64 code pairs keep a row code in one byte and a wide block (C W 36 bytes) small next to the chunk; a
-    // father whose op would outgrow the chunk keeps its second cherry as it is.  The fathers stay binary, so every op with a
-    // wide tip is one of the binary shapes.  BPPGPU_W4C_FRONTIER=0 folds none (the program of the unfolded walk).
+    // program (descriptor words + chunk records) in the kernel-parameter block.  One rate class per CTA: a chunk holds one
+    // class's blocks, and the tables of all classes chunk the same way.
+    const int nc = e->ncodes, W = nc * nc, W3 = nc * nc * nc;
+    const int blk_int = 128, blk_tip = nc * 32, blk_wide = w4c_wide_block_bytes(W), blk_wide3 = w4c_wide_block_bytes(W3);
+    e->w4c_nw = C <= 4 ? 4 : 8;
+    if (const char* env = getenv("BPPGPU_WALK4_NW")) {
+      const int v = atoi(env);
+      if ((v == 4 || v == 8) && v >= C) e->w4c_nw = v;
+    }
+    // Folded subtrees: a cherry whose father is binary becomes a wide tip of the father (walk4c_kernels.cuh), its op leaves the
+    // walk.  So does a three-tip subtree: a binary node under a binary father whose sons are a folded cherry and a tip.
+    // ncodes^2 (ncodes^3) <= 64 keeps a row code in one byte.  A father whose op would outgrow the chunk keeps its second
+    // folded son as it is (a three-tip subtree falls back to its op over the folded cherry, a cherry to its op over two tips).
+    // The fathers stay binary, so every op with a wide tip is one of the binary shapes.  BPPGPU_W4C_FRONTIER=0 folds none
+    // (the program of the unfolded walk).
+    auto sons = [&](int n) { return e->child_off[n + 1] - e->child_off[n]; };
+    auto son = [&](int n, int j) { return e->children[e->child_off[n] + j]; };
+    auto is_tip = [&](int n) { return e->leaf_slot[n] >= 0; };
     e->w4c_cherry.assign(nn, 0);
-    if (W <= kW4cMaxWideCodes && !(getenv("BPPGPU_W4C_FRONTIER") && atoi(getenv("BPPGPU_W4C_FRONTIER")) == 0)) {
-      auto sons = [&](int n) { return e->child_off[n + 1] - e->child_off[n]; };
-      auto son = [&](int n, int j) { return e->children[e->child_off[n] + j]; };
-      auto cherry = [&](int n) { return sons(n) == 2 && e->leaf_slot[son(n, 0)] >= 0 && e->leaf_slot[son(n, 1)] >= 0; };
+    e->w4c_three.assign(nn, 0);
+    const bool fold = W <= kW4cMaxWideCodes && !(getenv("BPPGPU_W4C_FRONTIER") && atoi(getenv("BPPGPU_W4C_FRONTIER")) == 0);
+    if (fold) {
+      for (int f = 0; f < nn; ++f)
+        if (sons(f) == 2)
+          for (int j = 0; j < 2; ++j) {
+            const int n = son(f, j);
+            e->w4c_cherry[n] = sons(n) == 2 && is_tip(son(n, 0)) && is_tip(son(n, 1));
+          }
+      if (W3 <= kW4cMaxWideCodes)
+        for (int f = 0; f < nn; ++f)
+          if (sons(f) == 2)
+            for (int j = 0; j < 2; ++j) {
+              const int n = son(f, j);
+              e->w4c_three[n] = sons(n) == 2 && ((e->w4c_cherry[son(n, 0)] && is_tip(son(n, 1))) ||
+                                                 (is_tip(son(n, 0)) && e->w4c_cherry[son(n, 1)]));
+            }
+    }
+    std::vector<char> folded(nn, 0);
+    auto make_folded = [&]() { for (int n = 0; n < nn; ++n) folded[n] = e->w4c_cherry[n] || e->w4c_three[n]; };
+    make_folded();
+    // chunk geometry, per class: CH bytes of tables and max_tips tip-code rows of PPC = NW 32 PT bytes per ring stage.  The
+    // ring gets the shared memory that walk4c_min_ctas(4, NW) CTAs per SM leave after the stack planes at PT = 4, split
+    // between tables and code rows in the program's own ratio of table bytes to tips, so both fill together.
+    build_program(e, e->prog4c, false, true, &folded);
+    auto child_bytes = [&](const Child& ch) {
+      return ch.kind != CHILD_TIP ? blk_int : ch.idx >= 0 ? blk_tip : e->w4c_three[ch.pnode] ? blk_wide3 : blk_wide;
+    };
+    int CH = 0;
+    {
+      long long tbytes = 0, ntip = 0;
+      for (const Op& op : e->prog4c.ops)
+        for (int j = 0; j < op.nchild; ++j) {
+          const Child& ch = e->prog4c.childs[op.child_begin + j];
+          tbytes += child_bytes(ch);
+          ntip += ch.kind == CHILD_TIP;
+        }
+      const long long ppc4 = (long long)e->w4c_nw * 32 * 4;
+      const long long budget = std::min<long long>(200 * 1024, g_smem_per_sm / walk4c_min_ctas(4, e->w4c_nw) - 2048);
+      const long long stage = std::max<long long>(0, (budget - (long long)walk4c_smem_bytes(0, e->prog4c.nslots, 4, e->w4c_nw, 0)) / kW4cStages);
+      const long long per_tip = ntip > 0 ? (tbytes + ntip - 1) / ntip : 128;
+      e->w4c_max_tips = (int)std::max<long long>(1, std::min<long long>(kW4cMaxTipsPerChunk, stage / (ppc4 + per_tip)));
+      CH = (int)std::max<long long>(2048, (stage - e->w4c_max_tips * ppc4) & ~127LL);
+    }
+    if (const char* env = getenv("BPPGPU_WALK4_CH")) CH = std::max(1024, atoi(env) & ~127);
+    if (const char* env = getenv("BPPGPU_WALK4_MAXTIPS")) e->w4c_max_tips = std::max(1, std::min(kW4cMaxTipsPerChunk, atoi(env)));
+    if (fold) {
+      bool changed = false;
       for (int f = 0; f < nn; ++f) {
         if (sons(f) != 2) continue;
-        for (int j = 0; j < 2; ++j) e->w4c_cherry[son(f, j)] = cherry(son(f, j));
         for (int j = 1; j >= 0; --j) {
           int b = 0;
           for (int k = 0; k < 2; ++k) {
             const int ch = son(f, k);
-            b += e->w4c_cherry[ch] ? blk_wide : e->leaf_slot[ch] >= 0 ? blk_tip : blk_int;
+            b += e->w4c_three[ch] ? blk_wide3 : e->w4c_cherry[ch] ? blk_wide : is_tip(ch) ? blk_tip : blk_int;
           }
-          if (b > CH) e->w4c_cherry[son(f, j)] = 0;
+          if (b <= CH) break;
+          const int n = son(f, j);
+          if (e->w4c_three[n]) e->w4c_three[n] = 0;
+          else e->w4c_cherry[n] = 0;
+          changed = true;
         }
       }
+      for (int n = 0; n < nn; ++n)   // a three-tip subtree whose cherry was kept unfolded is no longer one
+        if (e->w4c_three[n] && !e->w4c_cherry[son(n, 0)] && !e->w4c_cherry[son(n, 1)]) e->w4c_three[n] = 0;
+      if (changed) {
+        make_folded();
+        build_program(e, e->prog4c, false, true, &folded);
+      }
     }
-    build_program(e, e->prog4c, false, true, &e->w4c_cherry);
-    auto child_bytes = [&](const Child& ch) { return ch.kind != CHILD_TIP ? blk_int : ch.idx >= 0 ? blk_tip : blk_wide; };
     int max_op = 0, max_tips_op = 0;
     bool ok = e->prog4c.nslots <= 63;
     for (const Op& op : e->prog4c.ops) {
@@ -830,44 +891,38 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
       max_tips_op = std::max(max_tips_op, nt);
       if (op.nchild > 6) ok = false;
     }
-    while (CH < max_op) CH *= 2;
-    e->w4c_max_tips = getenv("BPPGPU_WALK4_MAXTIPS") ? std::max(1, std::min(31, atoi(getenv("BPPGPU_WALK4_MAXTIPS")))) : kW4cMaxTipsPerChunk;
+    while (CH < max_op) CH += 128;
     e->w4c_max_tips = std::max(e->w4c_max_tips, max_tips_op);
-    if (e->w4c_max_tips > 31) ok = false;
-    // launch plan.  Patterns per thread PT = 4 / 2 / 1 run 2 / 3 / 4 CTAs (of NW warps, 32 PT NW / C patterns) per SM; measured
-    // on the 1024-taxon tree (ms per evaluation): 10.4 / 11.3 / 15.2 at 1M patterns, 1.47 / 1.56 / 1.98 at 125k -- PT = 4 wins at
-    // every size that fills the GPU, so the default is ONE segment at the widest PT that has enough CTAs.  A launch is a
-    // whole number of waves; BPPGPU_WALK4_PLAN=split walks k full waves at PT = 4 and the remainder with narrower CTAs
-    // (measured on 125k patterns: 1.483 vs 1.469 ms -- the partial last wave of wide CTAs already runs at one CTA per SM and
-    // is cheaper than a wave of narrow ones, so the split is not the default).  BPPGPU_WALK4_PT forces one segment.
-    e->w4c_nw = C <= 4 ? 4 : 8;
-    if (const char* env = getenv("BPPGPU_WALK4_NW")) {
-      const int v = atoi(env);
-      if ((v == 4 || v == 8) && v >= C) e->w4c_nw = v;
-    }
+    if (e->w4c_max_tips > kW4cMaxTipsPerChunk) ok = false;
+    // launch plan.  Patterns per thread PT = 4 / 2 / 1 run 2 / 3 / 4 CTAs (of NW warps, 32 PT NW patterns of one class) per SM;
+    // measured on the 1024-taxon tree (ms per evaluation): 10.4 / 11.3 / 15.2 at 1M patterns, 1.47 / 1.56 / 1.98 at 125k --
+    // PT = 4 wins at every size that fills the GPU, so the default is ONE segment at the widest PT that has enough CTAs.  A
+    // launch is a whole number of waves; BPPGPU_WALK4_PLAN=split walks k full waves at PT = 4 and the remainder with narrower
+    // CTAs (measured on 125k patterns: 1.483 vs 1.469 ms -- the partial last wave of wide CTAs already runs at one CTA per SM
+    // and is cheaper than a wave of narrow ones, so the split is not the default).  BPPGPU_WALK4_PT forces one segment.
     int forced_pt = 0;
     if (const char* env = getenv("BPPGPU_WALK4_PT")) {
       const int v = atoi(env);
       if (v >= 1 && v <= 4) forced_pt = v;
     }
-    auto fits = [&](int pt) { return walk4c_smem_bytes(CH, e->prog4c.nslots, C, pt, e->w4c_nw, e->w4c_max_tips) <= 200 * 1024; };
+    auto fits = [&](int pt) { return walk4c_smem_bytes(CH, e->prog4c.nslots, pt, e->w4c_nw, e->w4c_max_tips) <= 200 * 1024; };
     if (!fits(1)) ok = false;
     if (ok) {
-      const int G = e->w4c_nw / C;
-      auto ppc = [&](int pt) { return (long long)G * 32 * pt; };
+      // ppc: patterns of one block (C CTAs, one per class); a wave of `slots` CTAs covers slots / C blocks
+      auto ppc = [&](int pt) { return (long long)e->w4c_nw * 32 * pt; };
       auto ctas_per_sm = [&](int pt) {
-        const size_t smem = walk4c_smem_bytes(CH, e->prog4c.nslots, C, pt, e->w4c_nw, e->w4c_max_tips) + 1024;
+        const size_t smem = walk4c_smem_bytes(CH, e->prog4c.nslots, pt, e->w4c_nw, e->w4c_max_tips) + 1024;
         const int by_regs = e->w4c_nw == 8 ? (pt <= 2 ? 2 : 1) : (pt <= 1 ? 4 : pt <= 3 ? 3 : 2);   // walk4c_min_ctas + registers
         return std::max(1, std::min<int>(by_regs, (int)(227 * 1024 / smem)));
       };
       const double wave_ms[5] = {0, 0.287, 0.315, 0.36, 0.386};   // relative cost of one wave (only ratios matter)
-      auto waves = [&](long long n, int pt) { const long long ctas = (n + ppc(pt) - 1) / ppc(pt); const long long slots = (long long)g_sm_count * ctas_per_sm(pt); return (ctas + slots - 1) / slots; };
+      auto waves = [&](long long n, int pt) { const long long ctas = C * ((n + ppc(pt) - 1) / ppc(pt)); const long long slots = (long long)g_sm_count * ctas_per_sm(pt); return (ctas + slots - 1) / slots; };
       e->w4c_segs.clear();
       auto add_seg = [&](int pt, long long a, long long b) {
         if (b <= a) return;
         bppgpu_engine::W4cSeg sg{};
         sg.pt = pt; sg.pat0 = a; sg.pat_end = b;
-        sg.grid = (int)((b - a + ppc(pt) - 1) / ppc(pt));
+        sg.grid = (int)(C * ((b - a + ppc(pt) - 1) / ppc(pt)));
         e->w4c_segs.push_back(sg);
       };
       if (forced_pt) {
@@ -876,12 +931,13 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
         add_seg(pt, 0, N);
       } else if (N > 0 && !(getenv("BPPGPU_WALK4_PLAN") && !strncmp(getenv("BPPGPU_WALK4_PLAN"), "split", 5))) {
         int big = 4;
-        while (big > 1 && (!fits(big) || N < (long long)g_sm_count * ctas_per_sm(big) * ppc(big))) big >>= 1;   // at least one wave
+        while (big > 1 && (!fits(big) || N * C < (long long)g_sm_count * ctas_per_sm(big) * ppc(big))) big >>= 1;   // at least one wave
         add_seg(big, 0, N);
       } else if (N > 0) {
         int big = 4;
         while (big > 1 && !fits(big)) big >>= 1;
-        const long long per_wave = (long long)g_sm_count * ctas_per_sm(big) * ppc(big);   // patterns in one full wave of the wide CTAs
+        // patterns in one full wave of the wide CTAs, a whole number of blocks
+        const long long per_wave = std::max<long long>(1, (long long)g_sm_count * ctas_per_sm(big) / C) * ppc(big);
         double best = 1e300;
         long long best_k = 0;
         int best_pt = 1;
@@ -905,12 +961,12 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
       e->w4c_pt = e->w4c_segs.empty() ? 1 : e->w4c_segs[0].pt;
     }
     if (ok) {
-      W4cProgram& W = e->w4c_prog;
-      memset(&W, 0, sizeof(W));
+      W4cProgram& Wp = e->w4c_prog;
+      memset(&Wp, 0, sizeof(Wp));
       int nwords = 0, nchunks = 0, nops_in = 0, ntips_in = 0, tip0 = 0;
       size_t used = 0;
       auto close_chunk = [&]() {
-        if (nchunks < kW4cMaxChunks) W.chunk[nchunks] = (unsigned)tip0 | ((unsigned)ntips_in << 16) | ((unsigned)nops_in << 21);
+        if (nchunks < kW4cMaxChunks) Wp.chunk[nchunks] = (unsigned)tip0 | ((unsigned)ntips_in << 16) | ((unsigned)nops_in << 21);
         ++nchunks;
         tip0 += ntips_in;
         nops_in = ntips_in = 0;
@@ -933,14 +989,17 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
           const Child& cb2 = e->prog4c.childs[op.child_begin + 1];
           const int ka = kind4c(ca.kind), kb = kind4c(cb2.kind);
           const bool wa = ka == W4C_TIP && ca.idx < 0, wb = kb == W4C_TIP && cb2.idx < 0;
-          // a wide tip is consumed first (W4C_WA); two wide tips set both bits
+          const bool w3a = wa && e->w4c_three[ca.pnode], w3b = wb && e->w4c_three[cb2.pnode];
+          // a wide tip is consumed first (W4C_WA); two wide tips set both bits; W4C_W3A / W4C_W3B mark three-tip tables
           if (ka == W4C_TIP && kb == W4C_TIP) {
             shape = W4C_TT;
             if (wb && !wa) { order[0] = 1; order[1] = 0; }
             wide = (wa || wb ? (unsigned)W4C_WA : 0u) | (wa && wb ? (unsigned)W4C_WB : 0u);
+            if (wa) wide |= (w3a ? (unsigned)W4C_W3A : 0u) | (w3b ? (unsigned)W4C_W3B : 0u);
+            else if (w3b) wide |= (unsigned)W4C_W3A;
           }
-          else if (ka == W4C_TIP && kb == W4C_REG) { shape = W4C_TS; wide = wa ? (unsigned)W4C_WA : 0u; }
-          else if (ka == W4C_REG && kb == W4C_TIP) { shape = W4C_TS; order[0] = 1; order[1] = 0; wide = wb ? (unsigned)W4C_WA : 0u; }
+          else if (ka == W4C_TIP && kb == W4C_REG) { shape = W4C_TS; wide = (wa ? (unsigned)W4C_WA : 0u) | (w3a ? (unsigned)W4C_W3A : 0u); }
+          else if (ka == W4C_REG && kb == W4C_TIP) { shape = W4C_TS; order[0] = 1; order[1] = 0; wide = (wb ? (unsigned)W4C_WA : 0u) | (w3b ? (unsigned)W4C_W3A : 0u); }
           else if (ka == W4C_RSL && kb == W4C_REG) shape = W4C_JW;
           else if (ka == W4C_REG && kb == W4C_RSL) { shape = W4C_JW; order[0] = 1; order[1] = 0; }
           else if (ka == W4C_SLOT && kb == W4C_REG) { shape = W4C_JS; jslot = (unsigned)ca.idx; }
@@ -958,25 +1017,35 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
             d2 |= (unsigned)kind4c(ch.kind) << (2 * j);
             if (ch.kind == CHILD_SLOT) d2 |= (unsigned)ch.idx << (12 + 6 * nslot_tok++);
           }
-          if (shape == W4C_GENERIC && ch.kind == CHILD_TIP && ch.idx < 0) ok = false;   // (the fathers of cherries are binary)
+          if (shape == W4C_GENERIC && ch.kind == CHILD_TIP && ch.idx < 0) ok = false;   // (the fathers of folded nodes are binary)
           Pack4cBlock pb{};
           pb.kind = kind4c(ch.kind);
           pb.pnode = ch.pnode;
-          pb.son0 = pb.son1 = -1;
+          pb.son0 = pb.son1 = pb.gson0 = pb.gson1 = -1;
           pb.off = (long long)((size_t)nchunks * CH + used);
-          if (ch.kind == CHILD_TIP && ch.idx < 0) {
+          if (ch.kind == CHILD_TIP && ch.idx < 0 && e->w4c_three[ch.pnode]) {
+            const int s0 = son(ch.pnode, 0), s1 = son(ch.pnode, 1);
+            pb.kind = W4C_THREE;
+            pb.tip_first = is_tip(s0);
+            pb.son0 = pb.tip_first ? s1 : s0;   // the folded cherry
+            pb.son1 = pb.tip_first ? s0 : s1;   // the tip
+            pb.gson0 = son(pb.son0, 0);
+            pb.gson1 = son(pb.son0, 1);
+            const int lt = e->leaf_slot[pb.son1], la = e->leaf_slot[pb.gson0], lb = e->leaf_slot[pb.gson1];
+            e->w4c_tip_order.push_back(pb.tip_first ? make_int3(lt, la, lb) : make_int3(la, lb, lt));
+          } else if (ch.kind == CHILD_TIP && ch.idx < 0) {
             pb.kind = W4C_CHERRY;
-            pb.son0 = e->children[e->child_off[ch.pnode]];
-            pb.son1 = e->children[e->child_off[ch.pnode] + 1];
-            e->w4c_tip_order.push_back(make_int2(e->leaf_slot[pb.son0], e->leaf_slot[pb.son1]));
+            pb.son0 = son(ch.pnode, 0);
+            pb.son1 = son(ch.pnode, 1);
+            e->w4c_tip_order.push_back(make_int3(e->leaf_slot[pb.son0], e->leaf_slot[pb.son1], -1));
           } else if (ch.kind == CHILD_TIP) {
-            e->w4c_tip_order.push_back(make_int2(ch.idx, -1));
+            e->w4c_tip_order.push_back(make_int3(ch.idx, -1, -1));
           }
           e->w4c_blocks.push_back(pb);
           used += (size_t)child_bytes(ch);
         }
         if (nslot_tok > 3) ok = false;
-        if (nwords < kW4cMaxOps) W.desc[nwords] = make_uint2(d, d2);
+        if (nwords < kW4cMaxOps) Wp.desc[nwords] = make_uint2(d, d2);
         ++nwords;
         ++nops_in;
         ntips_in += nt;
@@ -985,9 +1054,11 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
       if (nwords > kW4cMaxOps || nchunks > kW4cMaxChunks || e->w4c_tip_order.size() > 65535) ok = false;
       e->w4c_nchunks = nchunks;
       e->w4c_CH = CH;
-      e->w4c_stream_bytes = (size_t)nchunks * CH;
+      e->w4c_stream_bytes = (size_t)C * nchunks * CH;
       e->w4c = ok;
+      // folded cherries, those inside a folded three-tip subtree included
       e->w4c_frontier_nodes = ok ? (int)std::count(e->w4c_cherry.begin(), e->w4c_cherry.end(), 1) : 0;
+      e->w4c_three_tip_nodes = ok ? (int)std::count(e->w4c_three.begin(), e->w4c_three.end(), 1) : 0;
     }
   }
   int rc = upload_program(e, e->prog);
@@ -1134,19 +1205,26 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
     BPP_CUDA(dev_alloc(e, &e->d_w4c_blocks, e->w4c_blocks.size()));
     BPP_CUDA(cudaMemcpy(e->d_w4c_blocks, e->w4c_blocks.data(), e->w4c_blocks.size() * sizeof(Pack4cBlock), cudaMemcpyHostToDevice));
     BPP_CUDA(dev_alloc(e, &e->d_w4c_tip_order, e->w4c_tip_order.size()));
-    BPP_CUDA(cudaMemcpy(e->d_w4c_tip_order, e->w4c_tip_order.data(), e->w4c_tip_order.size() * sizeof(int2), cudaMemcpyHostToDevice));
-    size_t codes_bytes = 0;
+    BPP_CUDA(cudaMemcpy(e->d_w4c_tip_order, e->w4c_tip_order.data(), e->w4c_tip_order.size() * sizeof(int3), cudaMemcpyHostToDevice));
+    size_t codes_bytes = 0, scr = 0;
     int parts = 0;
     for (auto& sg : e->w4c_segs) {
+      const size_t ppc = (size_t)e->w4c_nw * 32 * sg.pt;
       sg.codes_off = codes_bytes;
       sg.part0 = parts;
-      codes_bytes += (size_t)sg.grid * e->w4c_tip_order.size() * (size_t)(e->w4c_nw / C) * 32 * sg.pt;
+      sg.scr_off = scr;
+      codes_bytes += (size_t)(sg.grid / C) * e->w4c_tip_order.size() * ppc;
       codes_bytes = (codes_bytes + 127) & ~(size_t)127;
+      scr += (size_t)sg.grid * ppc;
       parts += sg.grid;
     }
     BPP_CUDA(dev_alloc(e, &e->d_codesC, codes_bytes + 128));
     BPP_CUDA(dev_alloc(e, &e->d_w4c_counter, 1));
     BPP_CUDA(cudaMemset(e->d_w4c_counter, 0, sizeof(unsigned)));
+    BPP_CUDA(dev_alloc(e, &e->d_w4c_block_counter, (size_t)parts / C));
+    BPP_CUDA(cudaMemset(e->d_w4c_block_counter, 0, std::max<size_t>(1, (size_t)parts / C) * sizeof(unsigned)));
+    BPP_CUDA(dev_alloc(e, &e->d_w4c_csum, scr));
+    BPP_CUDA(dev_alloc(e, &e->d_w4c_cexp, scr));
   }
   if ((e->path != PATH_WALK4 || e->keep) && e->path != PATH_POINTS)
     BPP_CUDA(dev_alloc(e, &e->d_tiptab, (size_t)e->pchunk * e->nl * C * e->ncodes * S));
@@ -1166,6 +1244,8 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
   BPP_CUDA(dev_alloc(e, &e->d_site_lnl, (size_t)e->npoints * N));
   const long long rows = N * C;
   e->n_partials = (int)std::max<long long>(1, std::max((rows + 127) / 128, (N + 255) / 256) + 1);
+  if (e->w4c)
+    for (const auto& sg : e->w4c_segs) e->n_partials = std::max(e->n_partials, sg.part0 + sg.grid);
   BPP_CUDA(dev_alloc(e, &e->d_partials, (size_t)e->n_partials));
   BPP_CUDA(dev_alloc(e, &e->d_partials2, (size_t)e->n_partials));
   BPP_CUDA(dev_alloc(e, &e->d_out, (size_t)e->npoints * (1 + 2 * nn)));
@@ -1244,7 +1324,7 @@ static int create_impl(const bppgpu_config* cfg, bppgpu_engine* e) {
 
   if (e->w4c) {
     for (int pt = 1; pt <= 4; ++pt) {   // opt in to the dynamic shared memory of every instantiation a plan may use
-      const size_t smem = walk4c_smem_bytes(e->w4c_CH, e->prog4c.nslots, C, pt, e->w4c_nw, e->w4c_max_tips);
+      const size_t smem = walk4c_smem_bytes(e->w4c_CH, e->prog4c.nslots, pt, e->w4c_nw, e->w4c_max_tips);
       if (smem > 200 * 1024) continue;
       int rc4 = walk4c_dispatch(e, pt, nullptr, 0, smem, nullptr, true);
       if (rc4) return rc4;
@@ -1817,6 +1897,7 @@ static int enqueue_prune(bppgpu_engine* e, int point, int pl, cudaStream_t st) {
     wp.ncodes = e->ncodes;
     wp.ntips = (int)e->w4c_tip_order.size();
     wp.wide_codes = e->ncodes * e->ncodes;
+    wp.wide3_codes = e->ncodes * e->ncodes * e->ncodes;
     wp.max_tips = e->w4c_max_tips;
     wp.flags = rflag;
     wp.rootfreq = rootfreq;
@@ -1835,7 +1916,10 @@ static int enqueue_prune(bppgpu_engine* e, int point, int pl, cudaStream_t st) {
       wp.pat0 = sg.pat0;
       wp.pat_end = sg.pat_end;
       wp.part0 = sg.part0;
-      int rc4 = walk4c_dispatch(e, sg.pt, &wp, sg.grid, walk4c_smem_bytes(e->w4c_CH, e->prog4c.nslots, C, sg.pt, e->w4c_nw, e->w4c_max_tips), st, false);
+      wp.block_counter = e->d_w4c_block_counter + sg.part0 / C;
+      wp.csum = e->d_w4c_csum + sg.scr_off;
+      wp.cexp = e->d_w4c_cexp + sg.scr_off;
+      int rc4 = walk4c_dispatch(e, sg.pt, &wp, sg.grid, walk4c_smem_bytes(e->w4c_CH, e->prog4c.nslots, sg.pt, e->w4c_nw, e->w4c_max_tips), st, false);
       if (rc4) return rc4;
       nparts += sg.grid;
       e->stats.kernel_launches++;
@@ -2658,9 +2742,9 @@ static int eval_impl(bppgpu_engine* e, unsigned want, cudaStream_t st, bool time
     if (e->w4c) {
       if (e->codesT_dirty && e->N > 0) {
         for (const auto& sg : e->w4c_segs) {
-          pack_codesC_kernel<<<(unsigned)sg.grid, 256, 0, st>>>(
+          pack_codesC_kernel<<<(unsigned)(sg.grid / C), 256, 0, st>>>(
               (const unsigned char*)e->d_codes, e->d_w4c_tip_order, (int)e->w4c_tip_order.size(), e->ncodes, e->N, sg.pat0, sg.pat_end,
-              (e->w4c_nw / C) * 32 * sg.pt, e->d_codesC + sg.codes_off);
+              e->w4c_nw * 32 * sg.pt, e->d_codesC + sg.codes_off);
           e->stats.kernel_launches++;
         }
         e->codesT_dirty = false;
@@ -2672,12 +2756,13 @@ static int eval_impl(bppgpu_engine* e, unsigned want, cudaStream_t st, bool time
           pk.branch_model = pa_bm + (size_t)(p0 + pl) * nn;
           pk.brlen = pa_brlen + (size_t)(p0 + pl) * nn;
           pk.rates = e->d_rates; pk.code_table = e->d_code_table; pk.C = C; pk.ncodes = e->ncodes;
+          pk.class_bytes = e->w4c_stream_bytes / C;
           pk.P = e->d_P + (size_t)pl * nn * C * SS;
           pk.stream = e->d_w4c_stream + (size_t)pl * e->w4c_stream_bytes;
           pt_pack4c_kernel<<<(unsigned)e->w4c_blocks.size(), 64, 0, st>>>(pk);
         } else {
           pack_stream4c_kernel<<<(unsigned)e->w4c_blocks.size(), 64, 0, st>>>(
-              e->d_w4c_blocks, e->d_P + (size_t)pl * nn * C * SS, e->d_code_table, C, e->ncodes,
+              e->d_w4c_blocks, e->d_P + (size_t)pl * nn * C * SS, e->d_code_table, C, e->ncodes, e->w4c_stream_bytes / C,
               e->d_w4c_stream + (size_t)pl * e->w4c_stream_bytes);
         }
       }
@@ -3364,6 +3449,12 @@ int bppgpu_eval_multi(bppgpu_engine* const* engines, int32_t n_engines, unsigned
 int bppgpu_get_frontier_nodes(bppgpu_engine* e, int32_t* out) {
   if (!e || !out) BPP_FAIL(BPPGPU_E_INVALID, "null argument");
   *out = e->w4c_frontier_nodes;
+  return BPPGPU_OK;
+}
+
+int bppgpu_get_three_tip_nodes(bppgpu_engine* e, int32_t* out) {
+  if (!e || !out) BPP_FAIL(BPPGPU_E_INVALID, "null argument");
+  *out = e->w4c_three_tip_nodes;
   return BPPGPU_OK;
 }
 

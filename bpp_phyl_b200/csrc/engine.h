@@ -117,21 +117,27 @@ struct bppgpu_engine {
   bool w4c = false;
   bppgpu::Program prog4c;                  // walk program whose leaf pushes use the register slot
   bppgpu::W4cProgram w4c_prog;             // descriptor words + chunk records (passed as a kernel parameter)
-  size_t w4c_stream_bytes = 0;             // nchunks * CH
+  size_t w4c_stream_bytes = 0;             // C * nchunks * CH: the stream of one point, [class][chunk][CH]
   // launch plan: the pattern list is walked in one or two segments -- full waves of the widest CTAs, then the remainder with
-  // narrower ones (fewer patterns per thread, more CTAs per SM) so that the last wave is short
-  struct W4cSeg { int pt; long long pat0, pat_end; int grid; size_t codes_off; int part0; };
+  // narrower ones (fewer patterns per thread, more CTAs per SM) so that the last wave is short.  grid = C x blocks.
+  struct W4cSeg { int pt; long long pat0, pat_end; int grid; size_t codes_off; int part0; size_t scr_off; };
   std::vector<W4cSeg> w4c_segs;
   std::vector<bppgpu::Pack4cBlock> w4c_blocks;
-  std::vector<int2> w4c_tip_order;          // code rows in consumption order: {leaf slot, -1} or a cherry's {son 0, son 1}
-  std::vector<char> w4c_cherry;            // [nn] node is a folded cherry: a wide tip of prog4c (BPPGPU_W4C_FRONTIER=0: none)
+  std::vector<int3> w4c_tip_order;          // code rows in consumption order: the leaf slots of a tip / folded subtree, -1 padded
+  std::vector<char> w4c_cherry;            // [nn] node is a folded cherry: a wide tip of prog4c or part of a folded three-tip
+                                           // subtree (BPPGPU_W4C_FRONTIER=0: none)
+  std::vector<char> w4c_three;             // [nn] node is a folded three-tip subtree: a wide tip of prog4c
   int w4c_frontier_nodes = 0;              // folded cherries of the walk4c program in use
+  int w4c_three_tip_nodes = 0;             // folded three-tip subtrees of the walk4c program in use
   int w4c_CH = 0, w4c_nchunks = 0, w4c_pt = 2, w4c_nw = 8, w4c_max_tips = 16;
-  unsigned char* d_w4c_stream = nullptr;   // [pchunk][nchunks][CH]
+  unsigned char* d_w4c_stream = nullptr;   // [pchunk][C][nchunks][CH]
   bppgpu::Pack4cBlock* d_w4c_blocks = nullptr;
-  int2* d_w4c_tip_order = nullptr;
-  unsigned* d_w4c_counter = nullptr;       // CTAs done in the current evaluation (reset by the last one)
-  unsigned char* d_codesC = nullptr;       // [grid][ntips][PPC] tip codes as the CTAs stage them
+  int3* d_w4c_tip_order = nullptr;
+  unsigned* d_w4c_counter = nullptr;       // blocks done in the current evaluation, times C (reset by the last one)
+  unsigned* d_w4c_block_counter = nullptr; // [blocks] class CTAs of a block done (reset by the last one)
+  double* d_w4c_csum = nullptr;            // [blocks][C][PPC] class terms of the root reduction
+  int* d_w4c_cexp = nullptr;               // [blocks][C][PPC] their exponents
+  unsigned char* d_codesC = nullptr;       // [blocks][ntips][PPC] tip codes as the CTAs stage them
   // CLV storage (one point at a time)
   double* d_keep = nullptr;  // [ni][N][C][S]
   int* d_keep_exp = nullptr; // [ni][N][C]

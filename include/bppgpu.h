@@ -336,6 +336,9 @@ int bppgpu_get_stats(bppgpu_engine* e, bppgpu_stats* out);
 /* DNA walk (value-only S = 4 engines): cherries folded into wide tip tables, i.e. evaluated once per tip-code pair instead of
  * once per pattern (0 when none is; BPPGPU_W4C_FRONTIER=0 at engine creation folds none) */
 int bppgpu_get_frontier_nodes(bppgpu_engine* e, int32_t* out);
+/* three-tip subtrees (a folded cherry and a tip under a binary node) folded into wide tip tables the same way; their cherries
+ * are counted by bppgpu_get_frontier_nodes too */
+int bppgpu_get_three_tip_nodes(bppgpu_engine* e, int32_t* out);
 
 /* ---- multi-GPU: site patterns shard, nothing else does (SURVEY 8e) ---------------------------------------------------
  * The pattern loop of RHomogeneousTreeLikelihood::computeSubtreeLikelihood (RHomogeneousTreeLikelihood.cpp:839-861) has no

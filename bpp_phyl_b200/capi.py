@@ -347,6 +347,35 @@ def pairwise_distances_timing():
     return tuple(x.value for x in v)
 
 
+def _any_address(a, ctype):
+    """(pointer, keep-alive) of a numpy array (host), a torch tensor (pageable, pinned or CUDA) or an int address."""
+    if isinstance(a, int):
+        return C.cast(C.c_void_p(a), C.POINTER(ctype)), None
+    if hasattr(a, "data_ptr"):
+        assert a.is_contiguous()
+        return C.cast(C.c_void_p(a.data_ptr()), C.POINTER(ctype)), a
+    return a.ctypes.data_as(C.POINTER(ctype)), a
+
+
+def bootstrap_weights(indices, n_patterns, n_replicates, seed, first=0, device=0, out=None, n_sites=None):
+    """bppgpu_bootstrap_weights: [n_replicates][n_patterns] uint32 pattern weights of bootstrap replicates first ..
+    first + n_replicates - 1 (draws with replacement of the sites; ``indices`` [n_sites] = site -> pattern, int64).
+    ``indices`` and ``out`` may be numpy arrays, torch tensors (pageable, pinned or CUDA) or int addresses (then give
+    ``n_sites``).  Returns ``out`` (a new numpy array when None)."""
+    if not isinstance(indices, int) and not hasattr(indices, "data_ptr"):
+        indices = np.ascontiguousarray(indices, np.int64)
+    if n_sites is None:
+        n_sites = len(indices)
+    if out is None:
+        out = np.zeros((n_replicates, n_patterns), np.uint32)
+    iptr, keep_i = _any_address(indices, C.c_int64)
+    optr, keep_o = _any_address(out, C.c_uint32)
+    _check(lib().bppgpu_bootstrap_weights(C.c_int(device), C.c_int64(n_sites), iptr, C.c_int64(n_patterns), C.c_int64(first),
+                                          C.c_int32(n_replicates), C.c_uint64(seed), optr))
+    del keep_i, keep_o
+    return out
+
+
 class Parsimony:
     """Owning wrapper of a ``bppgpu_parsimony*``: Fitch parsimony over resident tip sets, topology per call.
 
@@ -408,8 +437,57 @@ class Parsimony:
         _check(lib().bppgpu_parsimony_nni(self._h, C.c_int32(n), C.c_int32(root), *ptrs, _ptr(d, C.c_int64), C.byref(s)))
         return d, s.value
 
+    def set_replicate_weights(self, weights, n_replicates=None):
+        """bppgpu_parsimony_set_replicate_weights: [R][N] uint32 (numpy, torch tensor in any memory, or an int address with
+        ``n_replicates``); an empty array or R = 0 frees them."""
+        if not isinstance(weights, int) and not hasattr(weights, "data_ptr"):
+            weights = np.ascontiguousarray(weights, np.uint32).reshape(-1, self.N)
+        R = n_replicates if n_replicates is not None else len(weights)
+        ptr, keep = _any_address(weights, C.c_uint32) if R else (None, None)
+        _check(lib().bppgpu_parsimony_set_replicate_weights(self._h, C.c_int32(R), ptr))
+        del keep
+
+    def draw_replicate_weights(self, indices, n_replicates, seed, first=0):
+        """bppgpu_parsimony_draw_replicate_weights: the replicate weights drawn on the device (as bootstrap_weights)."""
+        if not hasattr(indices, "data_ptr"):
+            indices = np.ascontiguousarray(indices, np.int64)
+        ptr, keep = _any_address(indices, C.c_int64)
+        _check(lib().bppgpu_parsimony_draw_replicate_weights(self._h, C.c_int64(len(indices)), ptr, C.c_int64(first),
+                                                             C.c_int32(n_replicates), C.c_uint64(seed)))
+        del keep
+
+    @staticmethod
+    def _batch(rep, topologies):
+        """rep [E] and E topologies (child_offsets, children, root, leaf_row) sharing n_nodes and root -> C arguments"""
+        rep = np.ascontiguousarray(rep, np.int32)
+        off = np.ascontiguousarray(np.stack([np.asarray(t[0], np.int32) for t in topologies]))
+        ch = np.ascontiguousarray(np.stack([np.asarray(t[1], np.int32) for t in topologies]))
+        lr = np.ascontiguousarray(np.stack([np.asarray(t[3], np.int32) for t in topologies]))
+        keep = (rep, off, ch, lr)
+        return len(rep), off.shape[1] - 1, int(topologies[0][2]), keep, \
+            (_ptr(off, C.c_int32), _ptr(ch, C.c_int32), _ptr(lr, C.c_int32))
+
+    def score_replicates(self, rep, topologies, site_scores=False):
+        """bppgpu_parsimony_score_replicates: scores [E] int64 of topology e under replicate rep[e]'s weights, and with
+        site_scores=True also the per-pattern scores [E][N] uint32."""
+        E, n, root, keep, ptrs = self._batch(rep, topologies)
+        s = np.zeros(E, np.int64)
+        sc = np.empty((E, self.N), np.uint32) if site_scores else None
+        _check(lib().bppgpu_parsimony_score_replicates(self._h, C.c_int32(E), _ptr(keep[0], C.c_int32), C.c_int32(n),
+                                                       C.c_int32(root), *ptrs, _ptr(s, C.c_int64), _ptr(sc, C.c_uint32)))
+        return (s, sc) if site_scores else s
+
+    def nni_replicates(self, rep, topologies):
+        """bppgpu_parsimony_nni_replicates: (delta [E][n_nodes] int64, scores [E] int64)."""
+        E, n, root, keep, ptrs = self._batch(rep, topologies)
+        d = np.zeros((E, n), np.int64)
+        s = np.zeros(E, np.int64)
+        _check(lib().bppgpu_parsimony_nni_replicates(self._h, C.c_int32(E), _ptr(keep[0], C.c_int32), C.c_int32(n),
+                                                     C.c_int32(root), *ptrs, _ptr(d, C.c_int64), _ptr(s, C.c_int64)))
+        return d, s
+
     def last_ms(self):
-        """Device milliseconds of the passes of the last score / nni_deltas call."""
+        """Device milliseconds of the passes of the last score / nni call (single or batched), or of the last draw."""
         ms = C.c_double(0)
         _check(lib().bppgpu_parsimony_last_ms(self._h, C.byref(ms)))
         return ms.value

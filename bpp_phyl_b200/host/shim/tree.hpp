@@ -1,5 +1,9 @@
-// bppgpu shim (see ../bppgpu_shim.hpp): Node, TreeTemplate, TreeTemplateTools (TreeTemplate.h, TreeTemplateTools.h)
+// bppgpu shim (see ../bppgpu_shim.hpp): Node, TreeTemplate, TreeTemplateTools (TreeTemplate.h, TreeTemplateTools.h), and
+// BipartitionList / TreeTools::computeBootstrapValues (BipartitionList.h, TreeTools.h)
 #pragma once
+#include <cstdio>
+#include <set>
+
 #include "seq.hpp"
 
 namespace bppshim {
@@ -26,9 +30,17 @@ class Node {
   void setName(const std::string& n) { name_ = n; }
   void removeFather() { father_ = nullptr; }
   std::vector<Node*>& sons() { return sons_; }
+  // branch properties (the reference stores Clonable objects; here a number, e.g. TreeTools::BOOTSTRAP)
+  void setBranchProperty(const std::string& name, double v) { branchProps_[name] = v; }
+  bool hasBranchProperty(const std::string& name) const { return branchProps_.count(name) > 0; }
+  double getBranchProperty(const std::string& name) const {
+    auto it = branchProps_.find(name);
+    if (it == branchProps_.end()) throw Exception("PropertyNotFoundException: Node::getBranchProperty: " + name);
+    return it->second;
+  }
   Node* cloneSubtree() const {
     Node* n = new Node();
-    n->id_ = id_; n->hasLen_ = hasLen_; n->len_ = len_; n->name_ = name_;
+    n->id_ = id_; n->hasLen_ = hasLen_; n->len_ = len_; n->name_ = name_; n->branchProps_ = branchProps_;
     for (Node* s : sons_) n->addSon(s->cloneSubtree());
     return n;
   }
@@ -40,6 +52,7 @@ class Node {
   bool hasLen_;
   double len_;
   std::string name_;
+  std::map<std::string, double> branchProps_;
 };
 
 namespace TreeTemplateTools {
@@ -135,5 +148,71 @@ inline TreeTemplate<Node>* parenthesisToTree(const std::string& description) {
   return new TreeTemplate<Node>(parse_(description, pos));
 }
 }  // namespace TreeTemplateTools
+
+
+// BipartitionList (BipartitionList.h), minimal: one bitset per branch (every non-root node) over the leaves in sorted-name
+// order, normalised to the side without the first leaf, so that the two branches at the root of a rooted tree give one split
+// and the split does not depend on son order or rooting.
+class BipartitionList {
+ public:
+  explicit BipartitionList(const Tree& tree) {
+    names_ = tree.getLeavesNames();
+    std::sort(names_.begin(), names_.end());
+    std::map<std::string, size_t> bit;
+    for (size_t i = 0; i < names_.size(); ++i) bit[names_[i]] = i;
+    std::map<const Node*, std::vector<bool> > below;
+    for (Node* n : tree.getNodes()) {
+      std::vector<bool>& b = below[n];
+      b.assign(names_.size(), false);
+      if (n->isLeaf()) b[bit.at(n->getName())] = true;
+      for (size_t s = 0; s < n->getNumberOfSons(); ++s) {
+        const std::vector<bool>& c = below[n->getSon(s)];
+        for (size_t i = 0; i < b.size(); ++i) b[i] = b[i] || c[i];
+      }
+      if (!n->hasFather()) continue;
+      std::vector<bool> side = b;
+      if (side[0]) side.flip();
+      splits_.push_back(side);
+      nodes_.push_back(n);
+    }
+  }
+  const std::vector<std::string>& getElementNames() const { return names_; }
+  size_t getNumberOfBipartitions() const { return splits_.size(); }
+  const std::vector<bool>& getBitBipartition(size_t i) const { return splits_[i]; }
+  Node* getNode(size_t i) const { return nodes_[i]; }
+
+ private:
+  std::vector<std::string> names_;
+  std::vector<std::vector<bool> > splits_;
+  std::vector<Node*> nodes_;
+};
+
+namespace TreeTools {
+static const std::string BOOTSTRAP = "bootstrap";
+// computeBootstrapValues (TreeTools.cpp): for each internal branch of `tree`, the percentage of `trees` that contain its split,
+// rounded half up to `format` decimals, stored as the branch property BOOTSTRAP.  Leaf branches get none.
+inline void computeBootstrapValues(Tree& tree, const std::vector<Tree*>& trees, bool verbose = true, int format = 0) {
+  if (trees.empty()) throw Exception("TreeTools::computeBootstrapValues: no replicate trees");
+  const BipartitionList main(tree);
+  std::map<std::vector<bool>, size_t> count;
+  for (const Tree* t : trees) {
+    const BipartitionList bl(*t);
+    if (bl.getElementNames() != main.getElementNames())
+      throw Exception("TreeTools::computeBootstrapValues: a replicate tree has another leaf set");
+    std::set<std::vector<bool> > seen;
+    for (size_t i = 0; i < bl.getNumberOfBipartitions(); ++i)
+      if (seen.insert(bl.getBitBipartition(i)).second) ++count[bl.getBitBipartition(i)];
+  }
+  const double f = std::pow(10.0, format);
+  for (size_t i = 0; i < main.getNumberOfBipartitions(); ++i) {
+    Node* n = main.getNode(i);
+    if (n->isLeaf()) continue;
+    auto it = count.find(main.getBitBipartition(i));
+    const double v = 100.0 * (it == count.end() ? 0 : it->second) / trees.size();
+    n->setBranchProperty(BOOTSTRAP, std::floor(v * f + 0.5) / f);
+  }
+  if (verbose) std::printf("computeBootstrapValues: %zu trees, %zu branches\n", trees.size(), main.getNumberOfBipartitions());
+}
+}  // namespace TreeTools
 
 }  // namespace bppshim

@@ -172,9 +172,39 @@ int bppgpu_parsimony_score(bppgpu_parsimony* h, int32_t n_nodes, int32_t root, c
  * three-son root (BPPGPU_E_INVALID otherwise).                                                                               */
 int bppgpu_parsimony_nni(bppgpu_parsimony* h, int32_t n_nodes, int32_t root, const int32_t* child_offsets,
                          const int32_t* children, const int32_t* leaf_row, int64_t* delta, int64_t* score);
-/* device time (CUDA events) of the passes of the handle's last successful score / nni call */
+/* Bootstrap replicates (bppPars: SiteContainerTools::bootstrap, then a search per replicate; semantics in DESIGN §7b).
+ * bppgpu_parsimony_set_replicate_weights stores weights [n_replicates][n_patterns] (host, pinned or device memory) beside the
+ * handle's own weights, which it does not touch; n_replicates = 0 frees them.  bppgpu_parsimony_draw_replicate_weights fills
+ * them on the device with bppgpu_bootstrap_weights(h's device, n_sites, indices, h's n_patterns, first_replicate, n_replicates,
+ * seed), so that they never pass through the host.                                                                        */
+int bppgpu_parsimony_set_replicate_weights(bppgpu_parsimony* h, int32_t n_replicates, const uint32_t* weights);
+int bppgpu_parsimony_draw_replicate_weights(bppgpu_parsimony* h, int64_t n_sites, const int64_t* indices, int64_t first_replicate,
+                                            int32_t n_replicates, uint64_t seed);
+/* bppgpu_parsimony_score / _nni for a batch of n_entries topologies in one call: entry e is scored under replicate rep[e]'s
+ * weights (ids may repeat: several candidate trees of one replicate).  All entries share n_nodes and root; child_offsets
+ * [E][n_nodes + 1], children [E][n_nodes - 1], leaf_row [E][n_nodes].  score [E], site_scores [E][n_patterns] (may be NULL),
+ * delta [E][n_nodes].  Each entry is validated as the single calls validate one topology, and rep[e] must be below the stored
+ * number of replicates; a bad entry fails the whole call (BPPGPU_E_INVALID, its index in the message).                    */
+int bppgpu_parsimony_score_replicates(bppgpu_parsimony* h, int32_t n_entries, const int32_t* rep, int32_t n_nodes, int32_t root,
+                                      const int32_t* child_offsets, const int32_t* children, const int32_t* leaf_row,
+                                      int64_t* score, uint32_t* site_scores);
+int bppgpu_parsimony_nni_replicates(bppgpu_parsimony* h, int32_t n_entries, const int32_t* rep, int32_t n_nodes, int32_t root,
+                                    const int32_t* child_offsets, const int32_t* children, const int32_t* leaf_row,
+                                    int64_t* delta, int64_t* score);
+/* device time (CUDA events) of the passes of the handle's last successful score / nni call (single or batched), or of the
+ * sampler kernels of its last draw_replicate_weights */
 int bppgpu_parsimony_last_ms(bppgpu_parsimony* h, double* ms);
 int bppgpu_parsimony_destroy(bppgpu_parsimony* h);
+
+/* ---- bootstrap replicate weights (SiteContainerTools::bootstrap as pattern weights) ----
+ * weights [n_replicates][n_patterns]: how many times replicate first_replicate + r drew a site whose pattern is k, for
+ * n_sites draws with replacement; indices [n_sites] = SitePatterns::getIndices.  Draw j of replicate R: Philox4x32-10
+ * (Random123) with key (seed low 32 bits, seed high 32 bits) and counter (j low, j high, R, 0); u = x0 | x1 << 32; the site
+ * is floor(u * n_sites / 2^64).  A replicate depends only on (seed, its absolute index), so chunks equal one call.
+ * indices and weights: host, pinned or device memory of `device`.  BPPGPU_E_INVALID for n_sites < 1 or >= 2^32, an index
+ * outside [0, n_patterns), n_replicates < 1, or first_replicate + n_replicates > 2^32.                                   */
+int bppgpu_bootstrap_weights(int device, int64_t n_sites, const int64_t* indices, int64_t n_patterns, int64_t first_replicate,
+                             int32_t n_replicates, uint64_t seed, uint32_t* weights);
 
 /* ---- Interface 2: tree likelihood engine ----------------------------------- */
 typedef struct bppgpu_engine bppgpu_engine;

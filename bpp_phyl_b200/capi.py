@@ -376,6 +376,33 @@ def bootstrap_weights(indices, n_patterns, n_replicates, seed, first=0, device=0
     return out
 
 
+def simulate_event_counts(type_rates, lengths, n_sims, seed, first=0, device=0, count=None, sum=None):
+    """bppgpu_simulate_event_counts: stochastic-mapping tallies of paths first .. first + n_sims - 1 from every start state.
+    ``type_rates`` [T][S][S] (the off-diagonal rates of each event class), ``lengths`` [L].  Returns (count [L][S][S] uint64:
+    paths from a in state j at lengths[b], sum [L][S][S][T] uint64: their class-T events).  ``count`` and ``sum`` may be given
+    as numpy arrays or torch tensors (pageable, pinned or CUDA) of those shapes and are returned filled."""
+    R = np.ascontiguousarray(type_rates, np.float64)
+    T, S = R.shape[0], R.shape[1]
+    t = _f64(lengths).ravel()
+    if count is None:
+        count = np.empty((len(t), S, S), np.uint64)
+    if sum is None:
+        sum = np.empty((len(t), S, S, T), np.uint64)
+    cptr, keep_c = _any_address(count, C.c_uint64)
+    sptr, keep_s = _any_address(sum, C.c_uint64)
+    _check(lib().bppgpu_simulate_event_counts(C.c_int(device), C.c_int32(S), C.c_int32(T), _ptr(R), C.c_int64(len(t)), _ptr(t),
+                                              C.c_int64(first), C.c_int64(n_sims), C.c_uint64(seed), cptr, sptr))
+    del keep_c, keep_s
+    return count, sum
+
+
+def expected_events_timing():
+    """Device milliseconds of this thread's last simulate_event_counts / Engine.expected_events: (simulation, combination)."""
+    v = [C.c_double(0) for _ in range(2)]
+    _check(lib().bppgpu_expected_events_timing(*[C.byref(x) for x in v]))
+    return tuple(x.value for x in v)
+
+
 class Parsimony:
     """Owning wrapper of a ``bppgpu_parsimony*``: Fitch parsimony over resident tip sets, topology per call.
 
@@ -661,6 +688,17 @@ class Engine:
         jt = np.empty((self.N, self.S, self.S)) if joint else None
         _check(lib().bppgpu_get_marginal_posteriors(self._h, C.c_int32(point), C.c_int32(node), _ptr(post), _ptr(jt)))
         return post, jt
+
+    def expected_events(self, type_rates, n_sims, seed, point=0):
+        """ComputeChromosomeTransitionsExp by stochastic mapping: (expected [n_nodes][T] events of each class per branch,
+        unreached [n_nodes] posterior mass no path reached); the root's rows are 0.  ``type_rates`` [T][S][S]."""
+        R = np.ascontiguousarray(type_rates, np.float64)
+        T = R.shape[0]
+        ex = np.empty((self.nn, T))
+        un = np.empty(self.nn)
+        _check(lib().bppgpu_expected_events(self._h, C.c_int32(point), C.c_int32(T), _ptr(R), C.c_int64(n_sims), C.c_uint64(seed),
+                                            _ptr(ex), _ptr(un)))
+        return ex, un
 
     def ml_ancestral_states(self, point=0):
         """MLAncestralStateReconstruction: (states [n_nodes][N] int32, log joint likelihood of the best assignment [N])"""

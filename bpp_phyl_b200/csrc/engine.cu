@@ -8,6 +8,7 @@
 //   K4+K5 upper / deriv kernels               prefix pass and branch derivatives
 // on one stream; bppgpu_eval synchronises once at the end, bppgpu_eval_device not at all.
 #include "engine.h"
+#include "event_mapping.h"
 
 #include <algorithm>
 #include <cmath>
@@ -3066,32 +3067,30 @@ int bppgpu_get_node_posteriors(bppgpu_engine* e, int32_t point, int32_t node, do
   return BPPGPU_OK;
 }
 
-int bppgpu_get_marginal_posteriors(bppgpu_engine* e, int32_t point, int32_t node, double* post_out, double* joint_out) {
-  ENGINE_SYNC(e);
-  if (!e->keep) BPP_FAIL(BPPGPU_E_STATE, "bppgpu_get_marginal_posteriors needs BPPGPU_FLAG_KEEP_CLVS");
-  if (node < 0 || node >= e->nn || !post_out || point < 0 || point >= e->npoints) BPP_FAIL(BPPGPU_E_INVALID, "bad node / point or null out");
+namespace {
+
+// what bppgpu_get_marginal_posteriors and bppgpu_expected_events need resident: kept CLVs, an evaluation of `point`, not the
+// batched-points path
+int marginal_state(const bppgpu_engine* e, int32_t point, const char* who) {
+  if (!e->keep) BPP_FAIL(BPPGPU_E_STATE, "%s needs BPPGPU_FLAG_KEEP_CLVS", who);
   if (e->path == PATH_POINTS) BPP_FAIL(BPPGPU_E_STATE, "not available on the batched-points path");
   if (e->last_want == 0) BPP_FAIL(BPPGPU_E_STATE, "no evaluation yet");
   if (point != e->last_point) BPP_FAIL(BPPGPU_E_STATE, "CLVs resident are those of point %d", e->last_point);
+  return BPPGPU_OK;
+}
+
+// marginal_posterior_kernel for one node of the resident point into d_post [N][S] and d_joint [N][S][S] (may be null), on the
+// engine's stream.  A non-root node needs the prefix pass and its upper slab (BPPGPU_E_STATE otherwise).
+int launch_marginal(bppgpu_engine* e, int32_t point, int32_t node, double* d_post, double* d_joint) {
   const bool leaf = e->leaf_slot[node] >= 0, root = node == e->root;
-  if (root && joint_out) BPP_FAIL(BPPGPU_E_INVALID, "the root has no father: no joint posterior");
   const int S = e->S, C = e->C;
   const long long N = e->N;
-  if (N == 0) return BPPGPU_OK;
   const size_t clvn = (size_t)N * C * S, rows = (size_t)N * C;
   int uslab = -1;
   if (!root) {
     if (!(e->last_want & BPPGPU_EVAL_D1) || !e->d_upper) BPP_FAIL(BPPGPU_E_STATE, "upper CLVs exist after an eval with derivatives");
     uslab = e->upper_slab[node];
     if (uslab < 0) BPP_FAIL(BPPGPU_E_STATE, "the upper CLV of tip %d is not materialised at this problem size", node);
-  }
-  double *d_post = nullptr, *d_joint = nullptr;
-  auto cleanup = [&]() { cudaFree(d_post); cudaFree(d_joint); };
-  if (cudaMalloc(&d_post, (size_t)N * S * 8) != cudaSuccess ||
-      (joint_out && cudaMalloc(&d_joint, (size_t)N * S * S * 8) != cudaSuccess)) {
-    cleanup();
-    cudaGetLastError();
-    BPP_FAIL(BPPGPU_E_NOMEM, "out of device memory for the marginal posteriors of node %d", node);
   }
   MarginalParams mp{};
   mp.is_leaf = leaf; mp.is_root = root;
@@ -3113,15 +3112,136 @@ int bppgpu_get_marginal_posteriors(bppgpu_engine* e, int32_t point, int32_t node
   mp.rootfreq = e->d_rootfreq_used + (size_t)point * S;
   mp.probs = e->d_probs; mp.SR = e->d_SR; mp.rexp = e->d_rexp;
   mp.post = d_post; mp.joint = d_joint;
-  cudaStream_t st = e->stream;
   const int grid = (int)std::min<long long>((N * S + 127) / 128, (long long)g_sm_count * 32);
-  marginal_posterior_kernel<<<grid, 128, 0, st>>>(mp);
-  cudaError_t err = cudaGetLastError();
-  if (err == cudaSuccess) err = cudaMemcpyAsync(post_out, d_post, (size_t)N * S * 8, cudaMemcpyDeviceToHost, st);
+  marginal_posterior_kernel<<<grid, 128, 0, e->stream>>>(mp);
+  BPP_CUDA(cudaGetLastError());
+  return BPPGPU_OK;
+}
+
+}  // namespace
+
+int bppgpu_get_marginal_posteriors(bppgpu_engine* e, int32_t point, int32_t node, double* post_out, double* joint_out) {
+  ENGINE_SYNC(e);
+  if (!e->keep) BPP_FAIL(BPPGPU_E_STATE, "bppgpu_get_marginal_posteriors needs BPPGPU_FLAG_KEEP_CLVS");
+  if (node < 0 || node >= e->nn || !post_out || point < 0 || point >= e->npoints) BPP_FAIL(BPPGPU_E_INVALID, "bad node / point or null out");
+  int rc = marginal_state(e, point, "bppgpu_get_marginal_posteriors");
+  if (rc != BPPGPU_OK) return rc;
+  const bool root = node == e->root;
+  if (root && joint_out) BPP_FAIL(BPPGPU_E_INVALID, "the root has no father: no joint posterior");
+  const int S = e->S;
+  const long long N = e->N;
+  if (N == 0) return BPPGPU_OK;
+  double *d_post = nullptr, *d_joint = nullptr;
+  auto cleanup = [&]() { cudaFree(d_post); cudaFree(d_joint); };
+  if (cudaMalloc(&d_post, (size_t)N * S * 8) != cudaSuccess ||
+      (joint_out && cudaMalloc(&d_joint, (size_t)N * S * S * 8) != cudaSuccess)) {
+    cleanup();
+    cudaGetLastError();
+    BPP_FAIL(BPPGPU_E_NOMEM, "out of device memory for the marginal posteriors of node %d", node);
+  }
+  cudaStream_t st = e->stream;
+  rc = launch_marginal(e, point, node, d_post, d_joint);
+  if (rc != BPPGPU_OK) {
+    cleanup();
+    return rc;
+  }
+  cudaError_t err = cudaMemcpyAsync(post_out, d_post, (size_t)N * S * 8, cudaMemcpyDeviceToHost, st);
   if (err == cudaSuccess && joint_out) err = cudaMemcpyAsync(joint_out, d_joint, (size_t)N * S * S * 8, cudaMemcpyDeviceToHost, st);
   if (err == cudaSuccess) err = cudaStreamSynchronize(st);
   cleanup();
   BPP_CUDA(err);
+  return BPPGPU_OK;
+}
+
+int bppgpu_expected_events(bppgpu_engine* e, int32_t point, int32_t n_types, const double* type_rates, int64_t n_sims, uint64_t seed,
+                           double* expected, double* unreached) {
+  ENGINE_SYNC(e);
+  if (!expected || !type_rates) BPP_FAIL(BPPGPU_E_INVALID, "type_rates and expected must not be NULL");
+  if (point < 0 || point >= e->npoints) BPP_FAIL(BPPGPU_E_INVALID, "point %d out of range (0..%d)", point, e->npoints - 1);
+  int rc = marginal_state(e, point, "bppgpu_expected_events");
+  if (rc != BPPGPU_OK) return rc;
+  if (!(e->last_want & BPPGPU_EVAL_D1) || !e->d_upper) BPP_FAIL(BPPGPU_E_STATE, "upper CLVs exist after an eval with derivatives");
+  const int nn = e->nn, S = e->S;
+  for (int n = 0; n < nn; ++n)
+    if (n != e->root && e->upper_slab[n] < 0) BPP_FAIL(BPPGPU_E_STATE, "the upper CLV of tip %d is not materialised at this problem size", n);
+  // the joint posterior is summed over rate classes; the simulation runs one class
+  if (e->C != 1) BPP_FAIL(BPPGPU_E_INVALID, "expected events need one rate class, the engine has %d", e->C);
+  const int* bm = &e->h_branch_model[(size_t)point * nn];
+  const int first_node = e->root == 0 ? 1 : 0;
+  if (nn < 2) BPP_FAIL(BPPGPU_E_INVALID, "the tree has no branch");
+  for (int n = 0; n < nn; ++n)
+    if (n != e->root && bm[n] != bm[first_node])
+      BPP_FAIL(BPPGPU_E_INVALID, "the branches of point %d use different model slots (%d and %d)", point, bm[first_node], bm[n]);
+  // t_b as the P(t) kernels form it: model rate x (length x rates[0])
+  std::vector<double> len;
+  std::vector<int> branch(nn, -1);
+  for (int n = 0; n < nn; ++n) {
+    if (n == e->root) continue;
+    branch[n] = (int)len.size();
+    len.push_back(e->models[bm[n]].rate * (e->h_brlen[(size_t)point * nn + n] * e->h_rates[0]));
+  }
+  double* tm = event_timing();
+  tm[0] = tm[1] = 0;
+  EventTallies tl;
+  double sim_ms = 0;
+  rc = event_tallies(e->dev, e->stream, S, n_types, type_rates, (int64_t)len.size(), len.data(), 0, n_sims, seed, tl, &sim_ms);
+  if (rc != BPPGPU_OK) return rc;
+  const long long N = e->N;
+  const int T = n_types;
+  // the joint posteriors of a group of branches at a time (all of them when they fit 4 GB), then one combine launch per group
+  const size_t joint_bytes = (size_t)std::max<long long>(N, 1) * S * S * 8;
+  const int nb = (int)len.size();
+  const int group = (int)std::max<size_t>(1, std::min<size_t>((size_t)nb, ((size_t)4 << 30) / joint_bytes));
+  std::vector<int> rows, out_row;
+  for (int n = 0; n < nn; ++n)
+    if (n != e->root) {
+      rows.push_back(tl.row_of[(size_t)branch[n]]);
+      out_row.push_back(n);
+    }
+  double *d_post = nullptr, *d_joint = nullptr, *d_out = nullptr;
+  int* d_idx = nullptr;
+  auto cleanup = [&]() { cudaFree(d_post); cudaFree(d_joint); cudaFree(d_out); cudaFree(d_idx); };
+  if (cudaMalloc(&d_post, (size_t)std::max<long long>(N, 1) * S * 8) != cudaSuccess || cudaMalloc(&d_joint, joint_bytes * group) != cudaSuccess ||
+      cudaMalloc(&d_out, (size_t)nn * (T + 1) * 8) != cudaSuccess || cudaMalloc(&d_idx, (size_t)nb * 2 * sizeof(int)) != cudaSuccess) {
+    cleanup();
+    cudaGetLastError();
+    BPP_FAIL(BPPGPU_E_NOMEM, "out of device memory for the joint posteriors");
+  }
+  cudaStream_t st = e->stream;
+  cudaEvent_t ev[2];
+  BPP_CUDA(cudaEventCreate(&ev[0]));
+  BPP_CUDA(cudaEventCreate(&ev[1]));
+  struct EventGuard { cudaEvent_t* e; ~EventGuard() { cudaEventDestroy(e[0]); cudaEventDestroy(e[1]); } } evg{ev};
+  cudaError_t err = cudaMemsetAsync(d_out, 0, (size_t)nn * (T + 1) * 8, st);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(d_idx, rows.data(), (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(d_idx + nb, out_row.data(), (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
+  if (err == cudaSuccess) err = cudaEventRecord(ev[0], st);
+  for (int g0 = 0; g0 < nb && err == cudaSuccess && N > 0; g0 += group) {
+    const int g1 = std::min(nb, g0 + group);
+    for (int g = g0; g < g1; ++g) {
+      rc = launch_marginal(e, point, out_row[(size_t)g], d_post, d_joint + (size_t)(g - g0) * (joint_bytes / 8));
+      if (rc != BPPGPU_OK) {
+        cudaStreamSynchronize(st);
+        cleanup();
+        return rc;
+      }
+    }
+    err = event_combine(st, tl, g1 - g0, d_idx + g0, d_joint, e->d_weights, N, d_idx + nb + g0, d_out);
+  }
+  if (err == cudaSuccess) err = cudaEventRecord(ev[1], st);
+  std::vector<double> out((size_t)nn * (T + 1));
+  if (err == cudaSuccess) err = cudaMemcpyAsync(out.data(), d_out, out.size() * 8, cudaMemcpyDeviceToHost, st);
+  if (err == cudaSuccess) err = cudaStreamSynchronize(st);
+  float ms = 0;
+  if (err == cudaSuccess) err = cudaEventElapsedTime(&ms, ev[0], ev[1]);
+  cleanup();
+  BPP_CUDA(err);
+  for (int n = 0; n < nn; ++n) {
+    for (int t = 0; t < T; ++t) expected[(size_t)n * T + t] = out[(size_t)n * (T + 1) + t];
+    if (unreached) unreached[n] = out[(size_t)n * (T + 1) + T];
+  }
+  tm[0] = sim_ms;
+  tm[1] = ms;
   return BPPGPU_OK;
 }
 

@@ -28,6 +28,7 @@
 // Random123) with key (seed lo, seed hi) and counter (j lo, j hi, R, 0); u = x0 | x1 << 32 draws site floor(u * n_sites / 2^64).
 #include "common.cuh"
 #include "bppgpu.h"
+#include "philox.cuh"
 #include "staging.h"
 
 #include <algorithm>
@@ -193,23 +194,6 @@ __global__ void __launch_bounds__(kThreads) pars_pre_kernel(const Entry* __restr
 }
 
 // ---- bootstrap replicate weights ----------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    if (r) {
-      k0 += 0x9E3779B9u;
-      k1 += 0xBB67AE85u;
-    }
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-    const uint32_t x0 = hi1 ^ c[1] ^ k0, x2 = hi0 ^ c[3] ^ k1;
-    c[0] = x0;
-    c[1] = lo1;
-    c[2] = x2;
-    c[3] = lo0;
-  }
-}
-
 __global__ void boot_check_kernel(const int64_t* __restrict__ idx, long long n_sites, long long n_patterns, int* __restrict__ bad) {
   for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n_sites; j += (long long)gridDim.x * blockDim.x)
     if (idx[j] < 0 || idx[j] >= n_patterns) atomicOr(bad, 1);

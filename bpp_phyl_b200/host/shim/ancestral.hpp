@@ -165,6 +165,55 @@ class MarginalNonRevAncestralStateReconstruction {
   std::unique_ptr<std::map<int, std::map<size_t, VVdouble> > > jointProbabilities_;
 };
 
+// ---- expected numbers of chromosome-number events per branch (fork) ----------------------------------------------------------
+// ChromosomeNumberMng::computeExpectations: ComputeChromosomeTransitionsExp built from the fitted likelihood and its model.
+// Stochastic mapping (Mayrose et al. 2010) with the estimator of bppgpu_expected_events (DESIGN §7b): numOfSimulations paths per
+// start state over the branch lengths, combined with the (node, father) joint posteriors of
+// MarginalNonRevAncestralStateReconstruction, which stay on the device.  The reference's random stream is not reproduced; a
+// run depends only on the seed.  runSimulations does the device call (simulation and combination together);
+// computeExpectationPerType forms the tree totals.
+class ComputeChromosomeTransitionsExp {
+ public:
+  typedef ChromosomeSubstitutionModel::typeOfTransition typeOfTransition;
+  ComputeChromosomeTransitionsExp(AbstractHomogeneousTreeLikelihood* tl, const ChromosomeSubstitutionModel* model)
+      : likelihood_(tl), model_(model) {}
+
+  void runSimulations(int numOfSimulations, uint64_t seed = 0) {
+    if (numOfSimulations < 1) throw Exception("ComputeChromosomeTransitionsExp::runSimulations: need at least one simulation");
+    likelihood_->getExpectedEvents(ChromosomeSubstitutionModel::NUMTYPES, model_->getTypeRates(), numOfSimulations, seed, expected_,
+                                   unreached_);
+    totals_.clear();
+  }
+  void computeExpectationPerType() {
+    if (expected_.empty()) throw Exception("ComputeChromosomeTransitionsExp: runSimulations first");
+    totals_.assign(ChromosomeSubstitutionModel::NUMTYPES, 0.0);
+    for (size_t n = 0; n < unreached_.size(); ++n)
+      for (int t = 0; t < ChromosomeSubstitutionModel::NUMTYPES; ++t) totals_[(size_t)t] += expected_[n * ChromosomeSubstitutionModel::NUMTYPES + (size_t)t];
+  }
+  // expected number of class-`type` events on the branch above nodeId (0 at the root)
+  double getExpectation(int nodeId, int type) const {
+    require();
+    return expected_.at((size_t)nodeId * ChromosomeSubstitutionModel::NUMTYPES + (size_t)type);
+  }
+  // the tree's expected number of class-`type` events (computeExpectationPerType)
+  double getTotalExpectation(int type) const {
+    if (totals_.empty()) throw Exception("ComputeChromosomeTransitionsExp: computeExpectationPerType first");
+    return totals_.at((size_t)type);
+  }
+  // posterior mass of the branch above nodeId whose (father, node) states no path reached: it contributes nothing to the
+  // expectations, so a large value asks for more simulations
+  double getUnreachedMass(int nodeId) const {
+    require();
+    return unreached_.at((size_t)nodeId);
+  }
+
+ private:
+  void require() const { if (expected_.empty()) throw Exception("ComputeChromosomeTransitionsExp: runSimulations first"); }
+  AbstractHomogeneousTreeLikelihood* likelihood_;   // not owned
+  const ChromosomeSubstitutionModel* model_;         // not owned
+  Vdouble expected_, unreached_, totals_;
+};
+
 // Likelihood/RNonHomogeneousMixedTreeLikelihood.{h,cpp}: mixed models on groups of branches.  The reference expands the set into one
 // RNonHomogeneousTreeLikelihood per site path ("hyper-node") and adds their site likelihoods with the path probabilities
 // (RNonHomogeneousMixedTreeLikelihood.cpp: getLikelihoodForASite = sum_paths p_path L_path); here every path is one point of a

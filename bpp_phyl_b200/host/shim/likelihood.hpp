@@ -362,6 +362,18 @@ class AbstractHomogeneousTreeLikelihood {
             for (size_t y = 0; y < S; ++y) (*joint)[i][x][y] = jb[(i * S + x) * S + y];
     }
   }
+  // ComputeChromosomeTransitionsExp's estimator on the device (bppgpu_expected_events): expected [node][type] = expected number of
+  // events of each class of typeRates [nTypes][S][S] on the branch above each node, unreached [node] = posterior mass no path
+  // reached; nSims paths per start state.  The joint posteriors never leave the device.
+  void getExpectedEvents(int nTypes, const std::vector<double>& typeRates, int64_t nSims, uint64_t seed, Vdouble& expected,
+                         Vdouble& unreached) const {
+    requireInit();
+    ensureDerivativePass();
+    expected.assign(nodes_.size() * (size_t)nTypes, 0.0);
+    unreached.assign(nodes_.size(), 0.0);
+    check(bppgpu_expected_events(engine_, 0, nTypes, typeRates.data(), nSims, seed, expected.data(), unreached.data()),
+          "ComputeChromosomeTransitionsExp");
+  }
   // MLAncestralStateReconstruction's result (fork): states[node][distinct site] of the joint ML assignment, computed on the
   // device with the transition probabilities and root frequencies of the last evaluation; bestLogLik[i] = its log joint likelihood
   void getJointMLAncestralStates(std::vector<std::vector<size_t> >& states, Vdouble* bestLogLik = nullptr) const {

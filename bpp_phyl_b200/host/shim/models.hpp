@@ -631,6 +631,16 @@ class ChromosomeSubstitutionModel : public AbstractSubstitutionModel {
     else throw ParameterNotFoundException(name);
     update();
   }
+  // event classes of ComputeChromosomeTransitionsExp, in the order of their rate terms in update()
+  enum typeOfTransition { GAIN_T = 0, LOSS_T = 1, DUPL_T = 2, DEMIPLOIDY_T = 3, BASENUM_T = 4, NUMTYPES = 5 };
+  // the generator's off-diagonal split by the rate term that produced it: [NUMTYPES][S][S], zero diagonal.  Added in class order
+  // the five matrices give getGenerator()'s off-diagonal bit for bit (what bppgpu_expected_events takes as type_rates).
+  std::vector<double> getTypeRates() const {
+    const size_t n = size_;
+    std::vector<double> R(NUMTYPES * n * n, 0.0);
+    forEachRateTerm([&](int t, int r, int c, double v) { R[((size_t)t * n + (size_t)r) * n + (size_t)c] += v; });
+    return R;
+  }
 
  private:
   double rate_(int i, double c, double lin) const {  // getRate (:504-526)
@@ -639,33 +649,40 @@ class ChromosomeSubstitutionModel : public AbstractSubstitutionModel {
     if (lin == IgnoreParam) return total;
     return rc_ == LINEAR ? total + lin * (i - 1) : total * std::exp(lin * (i - 1));
   }
-  void update() {
-    const int mn = (int)chr_->getMin(), mx = (int)chr_->getMax(), n = (int)size_;
-    for (int i = 0; i < n; ++i)
-      for (int j = 0; j < n; ++j) generator_(i, j) = 0.0;
+  // every rate term of the generator in the order update() adds them: add(class, row, column, rate), class 0..4 = gain, loss,
+  // dupl, demi, baseNum.  A clamped jump keeps its class; the two demi / 2 targets at odd i are both demi.
+  template <class F>
+  void forEachRateTerm(F add) const {
+    const int mn = (int)chr_->getMin(), mx = (int)chr_->getMax();
     const double demi = demi_ == DemiEqualDupl ? dupl_ : demi_;
     for (int i = mn; i <= mx; ++i) {
       const int r = i - mn;
-      if (i + 1 <= mx) generator_(r, r + 1) += rate_(i, gain_, gainR_);
-      if (i - 1 >= mn) generator_(r, r - 1) += rate_(i, loss_, lossR_);
-      if (2 * i <= mx) generator_(r, 2 * i - mn) += rate_(i, dupl_, duplR_);
-      else if (i != mx) generator_(r, mx - mn) += rate_(i, dupl_, duplR_);
+      if (i + 1 <= mx) add(GAIN_T, r, r + 1, rate_(i, gain_, gainR_));
+      if (i - 1 >= mn) add(LOSS_T, r, r - 1, rate_(i, loss_, lossR_));
+      if (2 * i <= mx) add(DUPL_T, r, 2 * i - mn, rate_(i, dupl_, duplR_));
+      else if (i != mx) add(DUPL_T, r, mx - mn, rate_(i, dupl_, duplR_));
       if (demi != IgnoreParam && i != mx) {  // :533-560
-        if (i % 2 == 0 && (int)(i * 1.5) <= mx) generator_(r, (int)(i * 1.5) - mn) += demi;
+        if (i % 2 == 0 && (int)(i * 1.5) <= mx) add(DEMIPLOIDY_T, r, (int)(i * 1.5) - mn, demi);
         else if (i % 2 != 0 && (int)std::ceil(i * 1.5) <= mx) {
-          if (i == 1) generator_(r, (int)std::ceil(i * 1.5) - mn) += demi;
+          if (i == 1) add(DEMIPLOIDY_T, r, (int)std::ceil(i * 1.5) - mn, demi);
           else {
-            generator_(r, (int)std::ceil(i * 1.5) - mn) += demi / 2;
-            generator_(r, (int)std::floor(i * 1.5) - mn) += demi / 2;
+            add(DEMIPLOIDY_T, r, (int)std::ceil(i * 1.5) - mn, demi / 2);
+            add(DEMIPLOIDY_T, r, (int)std::floor(i * 1.5) - mn, demi / 2);
           }
-        } else generator_(r, mx - mn) += demi;
+        } else add(DEMIPLOIDY_T, r, mx - mn, demi);
       }
       if (i < mx && baseNum_ != (int)IgnoreParam)  // :562-577
         for (int j = i + 1; j <= mx; ++j) {
-          if (j == mx) { if ((unsigned)(j - i) <= maxChrRange_) generator_(r, j - mn) += baseNumR_; }
-          else if ((j - i) % baseNum_ == 0 && (unsigned)(j - i) <= maxChrRange_) generator_(r, j - mn) += baseNumR_;
+          if (j == mx) { if ((unsigned)(j - i) <= maxChrRange_) add(BASENUM_T, r, j - mn, baseNumR_); }
+          else if ((j - i) % baseNum_ == 0 && (unsigned)(j - i) <= maxChrRange_) add(BASENUM_T, r, j - mn, baseNumR_);
         }
     }
+  }
+  void update() {
+    const int n = (int)size_;
+    for (int i = 0; i < n; ++i)
+      for (int j = 0; j < n; ++j) generator_(i, j) = 0.0;
+    forEachRateTerm([this](int, int r, int c, double v) { generator_(r, c) += v; });
     setDiagonal();
     updateMatrices(false);
     for (size_t i = 0; i < size_; ++i) freq_[i] = 1.0 / (double)size_;

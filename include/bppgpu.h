@@ -206,6 +206,27 @@ int bppgpu_parsimony_destroy(bppgpu_parsimony* h);
 int bppgpu_bootstrap_weights(int device, int64_t n_sites, const int64_t* indices, int64_t n_patterns, int64_t first_replicate,
                              int32_t n_replicates, uint64_t seed, uint32_t* weights);
 
+/* ---- stochastic mapping of event classes (ComputeChromosomeTransitionsExp; Mayrose et al. 2010) ----
+ * type_rates [n_types][S][S]: the off-diagonal rates of each event class (zero diagonal); summed over the classes they give the
+ * generator's off-diagonal (chromosome model: gain, loss, dupl, demi, baseNum).  Path n (first_sim <= n < first_sim + n_sims)
+ * from start state a draws step k from Philox4x32-10 with key (seed low 32 bits, seed high 32 bits) and counter (n, a, k, 0):
+ * u1 = ((x0 | x1 << 32) >> 11) + 1) 2^-53, waiting time -log(u1) / r_i with r_i = sum_T sum_j type_rates[T][i][j];
+ * v = ((x2 | x3 << 32) >> 11) 2^-53 r_i, and the event is the first (T, j), T-major and j ascending, whose running sum of rates
+ * exceeds v.  A state with r_i = 0 is absorbing.  A path runs until its time passes the longest length; length b reads the
+ * state and class counts after every event at time <= lengths[b].  Semantics in DESIGN §7b.
+ *   count [n_lengths][S][S]          count[b][a][j] = paths from a in state j at lengths[b]
+ *   sum   [n_lengths][S][S][n_types] sum[b][a][j][T] = their total number of class-T events
+ * A path depends only on (seed, a, n), so chunks of paths add up to one call.  type_rates, lengths, count and sum: host, pinned
+ * or device memory of `device`.  BPPGPU_E_INVALID for negative, non-finite or diagonal class rates, n_types outside 1..8,
+ * S outside 1..65535, a negative or non-finite length, n_sims < 1, or first_sim + n_sims > 2^32.                          */
+int bppgpu_simulate_event_counts(int device, int32_t n_states, int32_t n_types, const double* type_rates, int64_t n_lengths,
+                                 const double* lengths, int64_t first_sim, int64_t n_sims, uint64_t seed, uint64_t* count,
+                                 uint64_t* sum);
+/* device time of the calling thread's last successful bppgpu_simulate_event_counts or bppgpu_expected_events (CUDA events):
+ * simulation with the prefix pass over the tallies, and combination with the joint posteriors (0 for the former); either
+ * pointer may be NULL                                                                                                      */
+int bppgpu_expected_events_timing(double* sim_ms, double* combine_ms);
+
 /* ---- Interface 2: tree likelihood engine ----------------------------------- */
 typedef struct bppgpu_engine bppgpu_engine;
 
@@ -314,6 +335,18 @@ int bppgpu_get_node_posteriors(bppgpu_engine* e, int32_t point, int32_t node, do
  * is one pass.  Valid after an eval with BPPGPU_EVAL_D1 on an engine created with BPPGPU_FLAG_KEEP_CLVS (the root needs
  * the value pass only).                                                                                              */
 int bppgpu_get_marginal_posteriors(bppgpu_engine* e, int32_t point, int32_t node, double* posterior, double* joint);
+/* ComputeChromosomeTransitionsExp (fork; runSimulations + computeExpectationPerType): the expected number of events of each
+ * class on every branch, by stochastic mapping.  bppgpu_simulate_event_counts runs n_sims paths per start state (first_sim 0)
+ * over the point's branch lengths t_b = length x model rate x rates[0], and each branch combines its tallies with the joint
+ * posterior J_b[i][x][y] of bppgpu_get_marginal_posteriors, which stays on the device:
+ *   expected [n_nodes][n_types]  E_T(b) = sum_i w_i sum_{y, x: count[b][y][x] > 0} J_b[i][x][y] sum[b][y][x][T] / count[b][y][x]
+ *   unreached [n_nodes] or NULL   sum_i w_i sum_{count[b][y][x] = 0} J_b[i][x][y]: the posterior mass no path reached
+ * The root's rows are 0.  Sums run in a fixed order: a call is deterministic.  BPPGPU_E_INVALID for more than one rate class,
+ * branches of the point on different model slots, and the inputs bppgpu_simulate_event_counts rejects; BPPGPU_E_STATE where
+ * bppgpu_get_marginal_posteriors returns it (BPPGPU_FLAG_KEEP_CLVS, an eval with BPPGPU_EVAL_D1, the resident point, not the
+ * batched-points path).  type_rates: host, pinned or device memory.                                                       */
+int bppgpu_expected_events(bppgpu_engine* e, int32_t point, int32_t n_types, const double* type_rates, int64_t n_sims,
+                           uint64_t seed, double* expected, double* unreached);
 /* MLAncestralStateReconstruction (fork; Likelihood/MLAncestralStateReconstruction.h, .cpp:6-188, leaf arrays
  * DRASRTreeLikelihoodData.cpp:265-300): joint maximum-likelihood reconstruction (Pupko et al. 2000) with the transition
  * probabilities and root frequencies of the last evaluation -- a max-product pass up the tree, the best root state of class 0,
